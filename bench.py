@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --steps K --warmup W     # the CPU implementation of the path
+    python bench.py --steps K --warmup W --dump-outputs DIR   # + what the last timed step returned, as .npy
 
 A *step* is one vectorised SalpRobotEnv.step() over every env of the rank (auto-reset on, one
 full breathing cycle = K_i in [0, 1348] physics substeps per env).  Workload at N = 1:
@@ -44,6 +45,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from
 
 FLOP_PER_SUBSTEP = 500.0            # SURVEY.md 8(d) "ALGORITHMIC work per unit"
 NOMINAL_FP32_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12
@@ -73,7 +75,14 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (rank 0's envs) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl cuda)")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -406,6 +415,8 @@ def run_cuda_arm(args):
     barrier()
     clocks = sampler.stop()
     batch.check()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, batch)
     step_kernel_name = batch.last_step_kernel          # what the launcher picked (salp_last_step_kernel)
     ms = max_over_ranks(ms)
     total_env_steps = sum_over_ranks(float(n * args.steps))
@@ -552,6 +563,32 @@ def run_cuda_arm(args):
         emit(line)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 64 << 20
+DUMP_OUTPUTS = ("obs", "reward", "terminated", "truncated", "terminal_obs", "substeps")
+
+
+def dump_outputs(out_dir, batch):
+    """What the last timed step handed its caller -- SalpBatch.step_device's (obs, reward, terminated,
+    truncated) and the terminal_obs / substeps beside them -- as float32 DIR/<name>.npy (flags and
+    substep counts are exact in float32).  Above DUMP_BYTES in all, the same rows of every array are
+    written for a fixed, seeded sample of envs, and their indices as env_index.npy."""
+    import numpy as np
+    import torch
+    torch.cuda.synchronize()
+    n = batch.num_envs
+    outs = {k: batch.dev[k].cpu().numpy().astype(np.float32) for k in DUMP_OUTPUTS}
+    row_bytes = sum(a[0].nbytes for a in outs.values())
+    budget = DUMP_BYTES - 128 * (len(outs) + 1)        # less one .npy header per file
+    if n * row_bytes > budget:
+        m = budget // (row_bytes + 8)
+        idx = np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+        outs = {k: a[idx] for k, a in outs.items()}
+        outs["env_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in outs.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def ncu_traffic(envs, precision):

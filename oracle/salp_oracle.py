@@ -6,8 +6,10 @@ import this module.  The product (grasp_lab_salp_b200/) never does.
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
 import os
 import subprocess
+import tempfile
 from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
@@ -17,25 +19,48 @@ from grasp_lab_salp_b200.params import (NUM_EPISODE_METRICS, SalpParams, default
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB_PATH = os.path.join(_HERE, "_build", "libsalp_oracle.so")
+_HASH_PATH = _LIB_PATH + ".hash"
 _lib = None
+_built = None
+
+
+def _digest() -> str:
+    h = hashlib.sha256()
+    for f in (os.path.join(_HERE, "salp_oracle.c"), os.path.join(_HERE, "..", "include", "salp_b200.h"),
+              os.path.join(_HERE, "Makefile")):
+        with open(f, "rb") as fh:
+            h.update(fh.read())
+    return h.hexdigest()
 
 
 def build(force: bool = False) -> str:
-    src = os.path.join(_HERE, "salp_oracle.c")
-    hdr = os.path.join(_HERE, "..", "include", "salp_b200.h")
-    stale = (not os.path.exists(_LIB_PATH)
-             or os.path.getmtime(_LIB_PATH) < max(os.path.getmtime(src), os.path.getmtime(hdr)))
-    if force or stale:
-        subprocess.run(["make", "-C", _HERE, "-B" if force else "-s"], check=True,
-                       stdout=subprocess.DEVNULL)
-    return _LIB_PATH
+    """Path of the oracle library, compiled first if missing or built from other sources (content
+    hash: a copied tree does not keep mtimes).  A read-only tree gets it in a temporary directory."""
+    global _built
+    if _built is not None and not force:
+        return _built
+    d = _digest()
+    if not force and os.path.exists(_LIB_PATH) and os.path.exists(_HASH_PATH):
+        with open(_HASH_PATH) as fh:
+            if fh.read() == d:
+                _built = _LIB_PATH
+                return _built
+    out = os.path.dirname(_LIB_PATH)
+    in_tree = os.access(out if os.path.isdir(out) else _HERE, os.W_OK)
+    if not in_tree:
+        out = tempfile.mkdtemp(prefix="salp_oracle_")
+    subprocess.run(["make", "-s", "-B", "-C", _HERE, f"OUT={out}"], check=True, stdout=subprocess.DEVNULL)
+    if in_tree:
+        with open(_HASH_PATH, "w") as fh:
+            fh.write(d)
+    _built = os.path.join(out, "libsalp_oracle.so")
+    return _built
 
 
 def lib():
     global _lib
     if _lib is None:
-        build()
-        L = C.CDLL(_LIB_PATH)
+        L = C.CDLL(build())
         L.orc_create.restype = C.c_void_p
         L.orc_create.argtypes = [C.POINTER(SalpParams), C.c_int64, C.c_uint64, C.c_int64]
         L.orc_destroy.argtypes = [C.c_void_p]

@@ -204,32 +204,30 @@ def _load_reference_callback():
     return mod.DetailedMetricsCallback
 
 
-def _reference_callback_reads_what_the_reference_env_would_give(cdll, rel):
-    """Drives SalpCudaVecEnv with the actions and scenes of a golden trace of the live reference and
-    feeds every step's (infos, dones) to the reference's DetailedMetricsCallback._on_step; what the
-    callback collected must be what the reference's own env + SB3 Monitor would have handed it
-    (recomputed here from the golden file): Monitor r / l, success / truncation, and the nine
-    navigation / action / velocity metrics of salp_robot_env.py:399-447.  The callback's
-    reward-component deques stay empty, as they do with the reference: it looks for `avg_r_track`
-    while the env emits `avg_rewards_track` (tensorboard_callback.py:114-123 vs salp_robot_env.py:441-445)."""
-    Callback = _load_reference_callback()
+EPISODE_KEYS = ("r", "l", "success", "truncated", "path_length", "direct_distance", "path_efficiency",
+                "final_distance", "initial_distance", "avg_compression", "avg_coast_time", "avg_nozzle_angle",
+                "avg_velocity")
+
+
+def _replay_reference_episodes(cdll, on_step):
+    """Drives SalpCudaVecEnv with the actions and scenes of a golden trace of the live reference
+    (ref_random.npz), calls on_step(infos, dones) after every step, and returns, in order of episode
+    end, what the reference's own env + SB3 Monitor hand out there (recomputed from the golden file):
+    Monitor r / l, success / truncation, and the nine navigation / action / velocity metrics of
+    salp_robot_env.py:399-447, as {key: [values]} over EPISODE_KEYS."""
     g = load_golden("ref_random.npz")
     acts = g["actions"]
     n, T, _ = acts.shape
     venv = SalpCudaVecEnv(n, golden_params(g, precision=PRECISION_F64), seed=0, info_mode="lazy", _cdll=cdll)
     venv.batch.set_scene_pool(g["targets"], g["obstacles"])
     venv.reset()
-    cb = Callback(log_freq=T)
     keys = [str(k) for k in g["metric_keys"]]
-    want = {k: [] for k in ("r", "l", "success", "truncated", "path_length", "direct_distance", "path_efficiency",
-                            "final_distance", "initial_distance", "avg_compression", "avg_coast_time",
-                            "avg_nozzle_angle", "avg_velocity")}
+    want = {k: [] for k in EPISODE_KEYS}
     ret = np.zeros(n)
     length = np.zeros(n, int)
     for t in range(T):
         obs, rew, dones, infos = venv.step(acts[:, t])
-        cb.locals = {"infos": infos, "dones": dones}
-        assert cb.on_step() is True
+        on_step(infos, dones)
         ret += g["reward"][:, t]
         length += 1
         ended = (g["terminated"][:, t] | g["truncated"][:, t]).astype(bool)
@@ -244,23 +242,73 @@ def _reference_callback_reads_what_the_reference_env_would_give(cdll, rel):
                 want[k].append(g["metrics"][i, t, keys.index(k)])
             ret[i] = 0.0
             length[i] = 0
+    venv.close()
     assert len(want["r"]) >= 20            # the trace does end episodes
+    return want
+
+
+def _assert_episode_values(got, want, rel):
+    for k, w in want.items():
+        # (the reference averages its float32 action lists in float32, salp_robot_env.py:420-427)
+        tol = 1e-6 if k in ("avg_compression", "avg_coast_time", "avg_nozzle_angle") else rel
+        np.testing.assert_allclose(np.array(list(got[k]), float), np.array(w, float), rtol=tol, atol=tol, err_msg=k)
+
+
+def _reference_callback_reads_what_the_reference_env_would_give(cdll, rel):
+    """Feeds every step's (infos, dones) of _replay_reference_episodes to the reference's
+    DetailedMetricsCallback._on_step; what the callback collected must be what the reference's own
+    env + SB3 Monitor would have handed it.  The callback's reward-component deques stay empty, as
+    they do with the reference: it looks for `avg_r_track` while the env emits `avg_rewards_track`
+    (tensorboard_callback.py:114-123 vs salp_robot_env.py:441-445)."""
+    Callback = _load_reference_callback()
+    T = load_golden("ref_random.npz")["actions"].shape[1]
+    cb = Callback(log_freq=T)
+
+    def on_step(infos, dones):
+        cb.locals = {"infos": infos, "dones": dones}
+        assert cb.on_step() is True
+
+    want = _replay_reference_episodes(cdll, on_step)
     got = {"r": cb.episode_rewards, "l": cb.episode_lengths, "success": cb.episode_successes,
            "truncated": cb.episode_truncations, "path_length": cb.episode_path_lengths,
            "direct_distance": cb.episode_direct_distances, "path_efficiency": cb.episode_efficiencies,
            "final_distance": cb.episode_final_distances, "initial_distance": cb.episode_initial_distances,
            "avg_compression": cb.episode_compressions, "avg_coast_time": cb.episode_coast_times,
            "avg_nozzle_angle": cb.episode_nozzle_angles, "avg_velocity": cb.episode_velocities}
-    for k, w in want.items():
-        # (the reference averages its float32 action lists in float32, salp_robot_env.py:420-427)
-        tol = 1e-6 if k in ("avg_compression", "avg_coast_time", "avg_nozzle_angle") else rel
-        np.testing.assert_allclose(np.array(list(got[k]), float), np.array(w, float), rtol=tol, atol=tol, err_msg=k)
+    _assert_episode_values(got, want, rel)
     assert len(cb.episode_r_tracks) == 0 and len(cb.episode_r_smooths) == 0
     # the aggregated TensorBoard scalars are logged from those deques (log_freq = T)
     assert cb.records["custom/navigation/success_rate"] == pytest.approx(np.mean(want["success"]))
     assert cb.records["custom/path/efficiency"] == pytest.approx(np.mean(want["path_efficiency"]), rel=rel)
     assert cb.records["reward/stats/total_mean"] == pytest.approx(np.mean(want["r"]), rel=rel)
-    venv.close()
+
+
+def _episode_infos_match_reference_trace(cdll, rel):
+    """What a metrics callback reads at each episode end, taken from the infos directly: Monitor r / l,
+    TimeLimit.truncated and the nine metrics must be what the reference handed out in its golden trace.
+    Needs nothing outside the repository, unlike the check through the reference's own callback."""
+    got = {k: [] for k in EPISODE_KEYS}
+
+    def on_step(infos, dones):
+        for i in np.flatnonzero(dones):
+            info = infos[i]
+            got["r"].append(info["episode"]["r"])
+            got["l"].append(info["episode"]["l"])
+            got["success"].append(0.0 if info["TimeLimit.truncated"] else 1.0)
+            got["truncated"].append(1.0 if info["TimeLimit.truncated"] else 0.0)
+            for k in EPISODE_KEYS[4:]:
+                got[k].append(info[k])
+
+    _assert_episode_values(got, _replay_reference_episodes(cdll, on_step), rel)
+
+
+def test_episode_infos_match_reference_trace_cpu():
+    _episode_infos_match_reference_trace(_cdll(False), 1e-8)
+
+
+@pytest.mark.gpu
+def test_episode_infos_match_reference_trace_gpu():
+    _episode_infos_match_reference_trace(_cdll(True), 1e-8)
 
 
 def test_reference_metrics_callback_on_the_vec_env_cpu():
