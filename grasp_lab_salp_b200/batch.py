@@ -232,14 +232,32 @@ class SalpBatch:
         return bufs["obs"]
 
     def step_device(self, actions, auto_reset: bool = True, sort_by_k: bool = False, extras: bool = False,
-                    pipeline=None, generic: bool = False, extra_flags: int = 0):
+                    pipeline=None, generic: bool = False, extra_flags: int = 0, out=None):
         """actions: float32 CUDA tensor [N,3] on this batch's device.  Asynchronous on the current
         torch stream.  Returns (obs, reward, terminated, truncated) device tensors (reused every
-        call); ``self.dev["terminal_obs"]`` etc. hold the rest."""
+        call); ``self.dev["terminal_obs"]`` etc. hold the rest.
+
+        out: optional dict of caller-owned tensors that receive this step's obs / reward / terminated /
+        truncated / terminal_obs instead of the batch's own buffers (any subset; e.g. views into a replay
+        ring, so that a step is stored with no copy).  Contiguous, on this device: obs and terminal_obs
+        float32 [N, D], reward float32 [N], terminated and truncated 1-byte (uint8 / bool) [N]."""
         import torch
         bufs = self._device_buffers()
         if actions.dtype != torch.float32 or not actions.is_cuda or tuple(actions.shape) != (self.num_envs, 3):
             raise ValueError("actions must be a float32 CUDA tensor of shape [num_envs, 3]")
+        if out:
+            n, d = self.num_envs, self.obs_dim
+            want = dict(obs=(n, d), terminal_obs=(n, d), reward=(n,), terminated=(n,), truncated=(n,))
+            bufs = dict(bufs)
+            for k, t in out.items():
+                if k not in want:
+                    raise ValueError(f"out: unknown buffer {k!r} (expected a subset of {sorted(want)})")
+                ok_dtype = t.dtype == torch.float32 if k in ("obs", "terminal_obs", "reward") else t.element_size() == 1
+                if not (ok_dtype and tuple(t.shape) == want[k] and t.is_contiguous() and t.is_cuda
+                        and t.device.index == self.device):
+                    raise ValueError(f"out[{k!r}] must be a contiguous {'float32' if k in ('obs', 'terminal_obs', 'reward') else 'uint8 / bool'} "
+                                     f"tensor of shape {list(want[k])} on cuda:{self.device}")
+                bufs[k] = t
         actions = actions.contiguous()
         io = self._io_dev
         io.actions = actions.data_ptr()

@@ -27,6 +27,7 @@ UNITS = {
     "salp_policy.cu": [],
     "salp_lstm.cu": [],                    # tcgen05 / TMA LSTM cell (needs the sm_100a target)
     "salp_lstm_train.cu": [],              # element-wise halves of the learner's LSTM step
+    "salp_sac.cu": [],                     # SAC actor: SIMT layer 1, tcgen05 layer 2, fused heads
 }
 
 

@@ -336,6 +336,28 @@ int salp_lstm_cell(const void* packed_dev, const float* bias_dev, const float* o
                    int64_t n, int32_t obs_dim, int32_t hidden, void* stream);
 int salp_lstm_check(void);
 
+/* ---- rollout-side SAC actor (stable-baselines3 SACPolicy as src/train_robot.py trains it: actor
+ * net_arch [256, 256], ReLU, squashed Gaussian; csrc/salp_sac.cu).  For N envs in one launch:
+ *     latent = ReLU(W2 ReLU(W1 obs + b1) + b2);  mu = Wmu latent + bmu;
+ *     log_std = clamp(Wls latent + bls, -20, 2);  u = mu + exp(log_std) noise  (noise_dev NULL: u = mu);
+ *     scaled = tanh(u) (what the replay stores);  env = low + (scaled + 1) / 2 (high - low) (what salp_step gets)
+ * Hidden size 256 and act_dim 3 are fixed; 1 <= obs_dim <= 64.  Layer 1 and the heads are fp32 (layer 1 an
+ * fmaf chain over the inputs in order, from b1); layer 2 runs on the tensor cores (tcgen05) with bf16 operands
+ * and fp32 accumulation.  Weights are torch nn.Linear layouts ([out, in], row-major, fp32, device memory).
+ * salp_sac_weight_bytes: size of packed_dev (< 0 for an invalid obs_dim).
+ * salp_sac_pack_weights: once per weight update; packed_dev 16-byte aligned.
+ * salp_sac_act: obs [N, obs_dim], noise [N, 3] standard normal or NULL, outputs [N, 3]; action_low / high:
+ *   host float[3].  Runs on the device that owns packed_dev.
+ * salp_sac_check: synchronises the current device; SALP_ERR_CUDA if a kernel gave up on a bounded barrier wait. */
+int64_t salp_sac_weight_bytes(int32_t obs_dim);
+int salp_sac_pack_weights(const float* w1, const float* b1, const float* w2, const float* b2,
+                          const float* w_mu, const float* b_mu, const float* w_log_std, const float* b_log_std,
+                          int32_t obs_dim, void* packed_dev, void* stream);
+int salp_sac_act(const void* packed_dev, int32_t obs_dim, const float* obs_dev, const float* noise_dev,
+                 int64_t n, const float* action_low, const float* action_high,
+                 float* env_action_dev, float* scaled_action_dev, void* stream);
+int salp_sac_check(void);
+
 /* ---- the element-wise halves of the LEARNER's LSTM step (RecurrentPPO update, BPTT; fp32, any hidden
  * size; csrc/salp_lstm_train.cu, used by grasp_lab_salp_b200/lstm_seq.py's autograd.Function) -----------
  * forward : gates [B, 4H] (torch order i, f, g, o; biases and both products already summed) ->
