@@ -71,6 +71,9 @@ PROTOTYPES = {
     "salp_sac_pack_weights": (C.c_int, [C.c_void_p] * 8 + [C.c_int32, C.c_void_p, C.c_void_p]),
     "salp_sac_act": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(C.c_float),
                                C.POINTER(C.c_float), C.c_void_p, C.c_void_p, C.c_void_p]),
+    "salp_sac_pack_weights_grouped": (C.c_int, [C.c_void_p] * 8 + [C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
+    "salp_sac_act_grouped": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64,
+                                       C.POINTER(C.c_float), C.POINTER(C.c_float), C.c_void_p, C.c_void_p, C.c_void_p]),
     "salp_sac_check": (C.c_int, []),
     "salp_lstm_pointwise_fwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32,
                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

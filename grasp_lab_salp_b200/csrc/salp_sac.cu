@@ -7,9 +7,12 @@
 //   a = tanh(u)                                              the scaled action the replay stores
 //   env_action = low + (a + 1) / 2 (high - low)              what salp_step gets
 //
-// salp_sac_act_kernel: persistent CTAs (at most one per SM: ~203 KB of shared memory), each looping
-// over 128-env tiles.  W2, packed once per weight update as a bf16 K-major image with the 128-byte
-// swizzle (salp_sac_pack_weights), is copied into shared memory once per CTA.  Per tile:
+// salp_sac_act_kernel: persistent CTAs (at most one per SM: ~203 KB of shared memory), each taking a
+// contiguous range of 128-env tiles.  W2, packed once per weight update as a bf16 K-major image with the
+// 128-byte swizzle (salp_sac_pack_weights), is copied into shared memory when a CTA starts on an agent.
+// One launch serves K agents (salp_sac_act_grouped; salp_sac_act is K = 1): agent k owns env rows
+// [k n, (k + 1) n) and packed image k, a tile never spans two agents, and the (agent, tile) list is
+// agent-major, so a CTA's range changes agent at most a few times.  Per tile:
 //   layer 1   SIMT fp32, two threads per env row (128 hidden units each): K is only obs_dim, no tile
 //             for a tensor core.  W1 is read through L1 (warp-uniform addresses: broadcasts).  ReLU'd h1
 //             goes to shared memory as bf16 in the swizzled A layout, then fence.proxy.async so the
@@ -45,6 +48,7 @@
 #define SAC_F32_FLOATS(D) (SAC_H * (D) + 2 * SAC_H + SAC_HEADS * SAC_H + SAC_HEADS)
 #define SAC_SMEM (SAC_W2_BYTES + SAC_A_BYTES + (SAC_HEADS * SAC_H + SAC_H + SAC_BM * SAC_HEADS + 8) * 4 + 1024)
 #define SAC_TMEM_COLS 256
+#define SAC_MAX_AGENTS 65535                    // grid.y of the pack kernel
 
 __device__ int salp_sac_status_word = 0;
 
@@ -52,16 +56,19 @@ struct SacBox {
   float lo[SAC_A], hi[SAC_A];
 };
 
-// one thread per element of W2 (into the swizzled bf16 image) or of the fp32 part
+// one thread per element of W2 (into the swizzled bf16 image) or of the fp32 part of agent blockIdx.y's image
+// (parameters stacked [K, ...], images `image_bytes` apart)
 __global__ void salp_sac_pack_kernel(const float* __restrict__ w1, const float* __restrict__ b1, const float* __restrict__ w2,
                                      const float* __restrict__ b2, const float* __restrict__ w_mu, const float* __restrict__ b_mu,
-                                     const float* __restrict__ w_ls, const float* __restrict__ b_ls, int D,
+                                     const float* __restrict__ w_ls, const float* __restrict__ b_ls, int D, int64_t image_bytes,
                                      uint8_t* __restrict__ packed) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t ag = blockIdx.y;
+  packed += ag * image_bytes;
   if (idx < SAC_H * SAC_H) {
     const int r = idx / SAC_H, k = idx % SAC_H;    // torch weight [out = r, in = k]: K-major already
     const uint32_t off = (uint32_t)(k / SAC_BK) * (SAC_H * 128) + sw128_offset(r, k % SAC_BK);
-    *reinterpret_cast<__nv_bfloat16*>(packed + off) = __float2bfloat16_rn(w2[idx]);
+    *reinterpret_cast<__nv_bfloat16*>(packed + off) = __float2bfloat16_rn(w2[ag * SAC_H * SAC_H + idx]);
     return;
   }
   int i = idx - SAC_H * SAC_H;
@@ -69,19 +76,20 @@ __global__ void salp_sac_pack_kernel(const float* __restrict__ w1, const float* 
   float* f = reinterpret_cast<float*>(packed + SAC_W2_BYTES);
   const int j = i;
   float x;
-  if (i < SAC_H * D) x = w1[i];
-  else if ((i -= SAC_H * D) < SAC_H) x = b1[i];
-  else if ((i -= SAC_H) < SAC_H) x = b2[i];
-  else if ((i -= SAC_H) < SAC_A * SAC_H) x = w_mu[i];
-  else if ((i -= SAC_A * SAC_H) < SAC_A * SAC_H) x = w_ls[i];
-  else if ((i -= SAC_A * SAC_H) < SAC_A) x = b_mu[i];
-  else x = b_ls[i - SAC_A];
+  if (i < SAC_H * D) x = w1[ag * SAC_H * D + i];
+  else if ((i -= SAC_H * D) < SAC_H) x = b1[ag * SAC_H + i];
+  else if ((i -= SAC_H) < SAC_H) x = b2[ag * SAC_H + i];
+  else if ((i -= SAC_H) < SAC_A * SAC_H) x = w_mu[ag * SAC_A * SAC_H + i];
+  else if ((i -= SAC_A * SAC_H) < SAC_A * SAC_H) x = w_ls[ag * SAC_A * SAC_H + i];
+  else if ((i -= SAC_A * SAC_H) < SAC_A) x = b_mu[ag * SAC_A + i];
+  else x = b_ls[ag * SAC_A + i - SAC_A];
   f[j] = x;
 }
 
 __global__ void __launch_bounds__(SAC_THREADS, 1)
-salp_sac_act_kernel(const uint8_t* __restrict__ packed, int D, const float* __restrict__ obs, const float* __restrict__ noise,
-                    int64_t n, SacBox box, float* __restrict__ env_action, float* __restrict__ scaled_action) {
+salp_sac_act_kernel(const uint8_t* __restrict__ packed, int64_t image_bytes, int num_agents, int D, const float* __restrict__ obs,
+                    const float* __restrict__ noise, int64_t n, SacBox box, float* __restrict__ env_action,
+                    float* __restrict__ scaled_action) {
   extern __shared__ uint8_t sac_smem_raw[];
   __shared__ __align__(8) uint64_t bar_acc;
   __shared__ uint32_t tmem_base_slot;
@@ -97,9 +105,6 @@ salp_sac_act_kernel(const uint8_t* __restrict__ packed, int D, const float* __re
   float* b2_s = bh_s + 8;
   float* part_s = b2_s + SAC_H;                                                 // [128][6]
 
-  const float* f32 = reinterpret_cast<const float*>(packed + SAC_W2_BYTES);
-  const float* w1 = f32;
-  const float* b1 = w1 + SAC_H * D;
   if (threadIdx.x == 0) {
     mbar_init(smem_u32(&bar_acc), 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -110,29 +115,42 @@ salp_sac_act_kernel(const uint8_t* __restrict__ packed, int D, const float* __re
                  : "memory");
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
-  {
-    const uint4* src = reinterpret_cast<const uint4*>(packed);
-    uint4* dst = reinterpret_cast<uint4*>(smem);
-    for (int i = threadIdx.x; i < SAC_W2_BYTES / 16; i += SAC_THREADS) dst[i] = __ldg(src + i);
-    const float* b2 = b1 + SAC_H;
-    const float* wh = b2 + SAC_H;
-    for (int i = threadIdx.x; i < SAC_HEADS * SAC_H; i += SAC_THREADS) wh_s[i] = wh[i];
-    if (threadIdx.x < SAC_HEADS) bh_s[threadIdx.x] = wh[SAC_HEADS * SAC_H + threadIdx.x];
-    b2_s[threadIdx.x] = b2[threadIdx.x];
-  }
-  fence_proxy_async_smem();                      // W2 was written through the generic proxy
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = tmem_base_slot;
   const uint32_t t_row = tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)(half * (SAC_H / 2));
-  const int64_t tiles = (n + SAC_BM - 1) / SAC_BM;
+  // this CTA's contiguous range of the agent-major (agent, tile) list
+  const int64_t tiles = (n + SAC_BM - 1) / SAC_BM, total = tiles * num_agents;
+  const int64_t t_begin = total * blockIdx.x / gridDim.x, t_end = total * (blockIdx.x + 1) / gridDim.x;
+  const float* w1 = nullptr;
+  const float* b1 = nullptr;
+  int64_t agent = -1;
   bool ok = true;
 
   uint32_t it = 0;
-  for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x, it++) {
-    const int64_t e = tile * SAC_BM + row;
-    const bool live = e < n;
+  for (int64_t t = t_begin; t < t_end; t++, it++) {
+    const int64_t ag = t / tiles, tile = t - ag * tiles;
+    if (ag != agent) {                           // this agent's W2, b2 and heads into shared memory
+      agent = ag;
+      const uint8_t* img = packed + ag * image_bytes;
+      w1 = reinterpret_cast<const float*>(img + SAC_W2_BYTES);
+      b1 = w1 + SAC_H * D;
+      __syncthreads();                           // the previous tile's epilogue is done with wh_s / b2_s
+      const uint4* src = reinterpret_cast<const uint4*>(img);
+      uint4* dst = reinterpret_cast<uint4*>(smem);
+      for (int i = threadIdx.x; i < SAC_W2_BYTES / 16; i += SAC_THREADS) dst[i] = __ldg(src + i);
+      const float* b2 = b1 + SAC_H;
+      const float* wh = b2 + SAC_H;
+      for (int i = threadIdx.x; i < SAC_HEADS * SAC_H; i += SAC_THREADS) wh_s[i] = wh[i];
+      if (threadIdx.x < SAC_HEADS) bh_s[threadIdx.x] = wh[SAC_HEADS * SAC_H + threadIdx.x];
+      b2_s[threadIdx.x] = b2[threadIdx.x];
+      fence_proxy_async_smem();                  // W2 was written through the generic proxy
+      __syncthreads();
+    }
+    const int64_t el = tile * SAC_BM + row;      // env row within the agent
+    const bool live = el < n;
+    const int64_t e = ag * n + el;
     // ---- layer 1: this thread's env row, hidden units 128 half .. + 127 -> bf16 A tile
     float x[SAC_MAX_D];
 #pragma unroll
@@ -242,24 +260,34 @@ int64_t salp_sac_weight_bytes(int32_t obs_dim) {
   return ((int64_t)SAC_W2_BYTES + 4 * (int64_t)SAC_F32_FLOATS(obs_dim) + 15) / 16 * 16;
 }
 
-int salp_sac_pack_weights(const float* w1, const float* b1, const float* w2, const float* b2, const float* w_mu,
-                          const float* b_mu, const float* w_log_std, const float* b_log_std, int32_t obs_dim,
-                          void* packed_dev, void* stream) {
+int salp_sac_pack_weights_grouped(const float* w1, const float* b1, const float* w2, const float* b2, const float* w_mu,
+                                  const float* b_mu, const float* w_log_std, const float* b_log_std, int32_t num_agents,
+                                  int32_t obs_dim, void* packed_dev, void* stream) {
   if (!w1 || !b1 || !w2 || !b2 || !w_mu || !b_mu || !w_log_std || !b_log_std || !packed_dev) return SALP_ERR_INVALID;
+  if (num_agents < 1 || num_agents > SAC_MAX_AGENTS) return SALP_ERR_INVALID;
   if (obs_dim < 1 || obs_dim > SAC_MAX_D || ((uintptr_t)packed_dev & 15)) return SALP_ERR_INVALID;
   DeviceOf guard(packed_dev);
   if (guard.dev < 0) return SALP_ERR_INVALID;
   const int total = SAC_H * SAC_H + SAC_F32_FLOATS(obs_dim);
-  salp_sac_pack_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
-      w1, b1, w2, b2, w_mu, b_mu, w_log_std, b_log_std, obs_dim, reinterpret_cast<uint8_t*>(packed_dev));
+  salp_sac_pack_kernel<<<dim3((total + 255) / 256, num_agents), 256, 0, (cudaStream_t)stream>>>(
+      w1, b1, w2, b2, w_mu, b_mu, w_log_std, b_log_std, obs_dim, salp_sac_weight_bytes(obs_dim),
+      reinterpret_cast<uint8_t*>(packed_dev));
   return cudaPeekAtLastError() == cudaSuccess ? SALP_OK : SALP_ERR_CUDA;
 }
 
-int salp_sac_act(const void* packed_dev, int32_t obs_dim, const float* obs_dev, const float* noise_dev, int64_t n,
-                 const float* action_low, const float* action_high, float* env_action_dev, float* scaled_action_dev,
-                 void* stream) {
+int salp_sac_pack_weights(const float* w1, const float* b1, const float* w2, const float* b2, const float* w_mu,
+                          const float* b_mu, const float* w_log_std, const float* b_log_std, int32_t obs_dim,
+                          void* packed_dev, void* stream) {
+  return salp_sac_pack_weights_grouped(w1, b1, w2, b2, w_mu, b_mu, w_log_std, b_log_std, 1, obs_dim, packed_dev, stream);
+}
+
+int salp_sac_act_grouped(const void* packed_dev, int32_t num_agents, int32_t obs_dim, const float* obs_dev,
+                         const float* noise_dev, int64_t envs_per_agent, const float* action_low, const float* action_high,
+                         float* env_action_dev, float* scaled_action_dev, void* stream) {
+  const int64_t n = envs_per_agent;
   if (!packed_dev || !obs_dev || !action_low || !action_high || !env_action_dev || !scaled_action_dev || n <= 0)
     return SALP_ERR_INVALID;
+  if (num_agents < 1 || num_agents > SAC_MAX_AGENTS) return SALP_ERR_INVALID;
   if (obs_dim < 1 || obs_dim > SAC_MAX_D || ((uintptr_t)packed_dev & 15)) return SALP_ERR_INVALID;
   DeviceOf guard(packed_dev);
   if (guard.dev < 0 || guard.dev >= 64) return SALP_ERR_INVALID;
@@ -276,11 +304,19 @@ int salp_sac_act(const void* packed_dev, int32_t obs_dim, const float* obs_dev, 
     box.lo[i] = action_low[i];
     box.hi[i] = action_high[i];
   }
-  const int64_t tiles = (n + SAC_BM - 1) / SAC_BM;
+  const int64_t tiles = (n + SAC_BM - 1) / SAC_BM * num_agents;
   const unsigned grid = (unsigned)(tiles < sms[guard.dev] ? tiles : sms[guard.dev]);
   salp_sac_act_kernel<<<grid, SAC_THREADS, SAC_SMEM, (cudaStream_t)stream>>>(
-      reinterpret_cast<const uint8_t*>(packed_dev), obs_dim, obs_dev, noise_dev, n, box, env_action_dev, scaled_action_dev);
+      reinterpret_cast<const uint8_t*>(packed_dev), salp_sac_weight_bytes(obs_dim), num_agents, obs_dim, obs_dev, noise_dev,
+      n, box, env_action_dev, scaled_action_dev);
   return cudaPeekAtLastError() == cudaSuccess ? SALP_OK : SALP_ERR_CUDA;
+}
+
+int salp_sac_act(const void* packed_dev, int32_t obs_dim, const float* obs_dev, const float* noise_dev, int64_t n,
+                 const float* action_low, const float* action_high, float* env_action_dev, float* scaled_action_dev,
+                 void* stream) {
+  return salp_sac_act_grouped(packed_dev, 1, obs_dim, obs_dev, noise_dev, n, action_low, action_high, env_action_dev,
+                              scaled_action_dev, stream);
 }
 
 /* synchronises the current device; SALP_ERR_CUDA if a kernel since the last call gave up on a barrier */

@@ -118,24 +118,27 @@ class SacCritic(nn.Module):
         return tuple(q(x) for q in self.q_networks)
 
 
-class SacActorB200:
-    """Rollout-side forward of a SacActor as ONE kernel (salp_sac_act, csrc/salp_sac.cu): layer 1 in
-    fp32 SIMT, layer 2 on the tensor cores with bf16 operands, heads, sampling, tanh and the Box
-    scaling fused.  Call `pack()` after every optimiser step.  CUDA only -- there is no CPU path."""
+class SacActorGroupB200:
+    """Rollout-side forward of K SacActors as ONE kernel (salp_sac_act_grouped, csrc/salp_sac.cu): layer 1 in
+    fp32 SIMT, layer 2 on the tensor cores with bf16 operands, heads, sampling, tanh and the Box scaling
+    fused.  `params` are the eight actor tensors (latent_pi.0 weight / bias, latent_pi.2, mu, log_std) stacked
+    [K, ...]; rows [k n, (k + 1) n) of a call belong to agent k.  Call `pack()` after every optimiser step.
+    CUDA only -- there is no CPU path."""
 
-    def __init__(self, actor: SacActor, action_low, action_high):
-        l1, l2 = actor.latent_pi[0], actor.latent_pi[2]
-        if l1.out_features != HIDDEN or l2.out_features != HIDDEN or actor.mu.out_features != ACT_DIM:
+    def __init__(self, params, action_low, action_high):
+        self.params = params
+        w1, w2, w_mu = params[0], params[2], params[4]
+        if w1.shape[1] != HIDDEN or tuple(w2.shape[1:]) != (HIDDEN, HIDDEN) or w_mu.shape[1] != ACT_DIM:
             raise ValueError(f"salp_sac_act is built for hidden size {HIDDEN} and {ACT_DIM} actions")
-        dev = l1.weight.device
+        dev = w1.device
         if dev.type != "cuda":
-            raise RuntimeError("SacActorB200 needs the actor's parameters on a CUDA device (no CPU path)")
+            raise RuntimeError(f"{type(self).__name__} needs the actor's parameters on a CUDA device (no CPU path)")
         self.lib = _lib.load()
-        self.actor, self.device, self.obs_dim = actor, dev, l1.in_features
-        nbytes = self.lib.salp_sac_weight_bytes(self.obs_dim)
-        if nbytes < 0:
+        self.device, self.num_agents, self.obs_dim = dev, w1.shape[0], w1.shape[2]
+        self.image_bytes = self.lib.salp_sac_weight_bytes(self.obs_dim)
+        if self.image_bytes < 0:
             raise ValueError(f"salp_sac_act supports obs_dim <= 64 (got {self.obs_dim})")
-        self.packed = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        self.packed = torch.empty(self.num_agents * self.image_bytes, dtype=torch.uint8, device=dev)
         self.lo = (C.c_float * 3)(*action_low)
         self.hi = (C.c_float * 3)(*action_high)
         self.pack()
@@ -143,31 +146,34 @@ class SacActorB200:
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
+    def _stacked(self):
+        return self.params
+
     def pack(self):
-        a = self.actor
-        ps = [a.latent_pi[0].weight, a.latent_pi[0].bias, a.latent_pi[2].weight, a.latent_pi[2].bias,
-              a.mu.weight, a.mu.bias, a.log_std.weight, a.log_std.bias]
+        ps = self._stacked()
         if any(p.dtype != torch.float32 or not p.is_contiguous() for p in ps):
             raise ValueError("the actor's parameters must be contiguous float32")
-        rc = self.lib.salp_sac_pack_weights(*[C.c_void_p(p.data_ptr()) for p in ps], self.obs_dim,
-                                            C.c_void_p(self.packed.data_ptr()), self._stream())
+        rc = self.lib.salp_sac_pack_weights_grouped(*[C.c_void_p(p.data_ptr()) for p in ps], self.num_agents,
+                                                    self.obs_dim, C.c_void_p(self.packed.data_ptr()), self._stream())
         if rc != 0:
             raise RuntimeError(f"salp_sac_pack_weights failed ({rc})")
 
     def act(self, obs, noise, env_action, scaled_action):
-        """obs [n, D] fp32; noise [n, 3] standard normal or None (deterministic: tanh(mu)); writes
-        env_action and scaled_action ([n, 3] fp32, contiguous, may be views into a replay ring)."""
+        """obs [n, D] fp32 (n a multiple of K); noise [n, 3] standard normal or None (deterministic: tanh(mu));
+        writes env_action and scaled_action ([n, 3] fp32, contiguous, may be views into a replay ring)."""
         n = obs.shape[0]
-        if not (n > 0 and obs.shape[1] == self.obs_dim and obs.dtype == torch.float32 and obs.is_contiguous()
-                and obs.device == self.device):
-            raise ValueError(f"obs must be a contiguous float32 [n, {self.obs_dim}] tensor on {self.device}")
+        if not (n > 0 and n % self.num_agents == 0 and obs.shape[1] == self.obs_dim and obs.dtype == torch.float32
+                and obs.is_contiguous() and obs.device == self.device):
+            raise ValueError(f"obs must be a contiguous float32 [n, {self.obs_dim}] tensor on {self.device}, "
+                             f"n a multiple of {self.num_agents}")
         for t in (noise, env_action, scaled_action):
             if t is not None and not (tuple(t.shape) == (n, 3) and t.dtype == torch.float32 and t.is_contiguous()
                                       and t.device == self.device):
                 raise ValueError(f"noise / actions must be contiguous float32 [{n}, 3] tensors on {self.device}")
-        rc = self.lib.salp_sac_act(C.c_void_p(self.packed.data_ptr()), self.obs_dim, C.c_void_p(obs.data_ptr()),
-                                   None if noise is None else C.c_void_p(noise.data_ptr()), n, self.lo, self.hi,
-                                   C.c_void_p(env_action.data_ptr()), C.c_void_p(scaled_action.data_ptr()), self._stream())
+        rc = self.lib.salp_sac_act_grouped(C.c_void_p(self.packed.data_ptr()), self.num_agents, self.obs_dim,
+                                           C.c_void_p(obs.data_ptr()), None if noise is None else C.c_void_p(noise.data_ptr()),
+                                           n // self.num_agents, self.lo, self.hi, C.c_void_p(env_action.data_ptr()),
+                                           C.c_void_p(scaled_action.data_ptr()), self._stream())
         if rc != 0:
             raise RuntimeError(f"salp_sac_act failed ({rc})")
         return env_action, scaled_action
@@ -177,21 +183,41 @@ class SacActorB200:
             raise RuntimeError("salp_sac_act: a kernel gave up waiting on its barrier")
 
 
+class SacActorB200(SacActorGroupB200):
+    """Rollout-side forward of one SacActor as ONE kernel (salp_sac_act, the K = 1 case of
+    SacActorGroupB200).  `pack()` reads the module's parameters again, so call it after every optimiser
+    step.  CUDA only -- there is no CPU path."""
+
+    def __init__(self, actor: SacActor, action_low, action_high):
+        self.actor = actor
+        super().__init__(self._stacked(), action_low, action_high)
+
+    def _stacked(self):
+        a = self.actor
+        return [p.detach().unsqueeze(0) for p in (a.latent_pi[0].weight, a.latent_pi[0].bias, a.latent_pi[2].weight,
+                                                   a.latent_pi[2].bias, a.mu.weight, a.mu.bias, a.log_std.weight,
+                                                   a.log_std.bias)]
+
+
 # ------------------------------------------------------------------------------------------------
 # SAC
 # ------------------------------------------------------------------------------------------------
+def _refuse_multi_rank(name):
+    try:
+        import torch.distributed as dist
+        if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+            raise RuntimeError(f"{name} is single-GPU: multi-GPU SAC (a replay per rank and a gradient all-reduce) "
+                               "is not implemented")
+    except ImportError:
+        pass
+
+
 class SAC:
     def __init__(self, env, config: SACConfig | None = None):
         self.env = env
         self.cfg = cfg = config or SACConfig()
         self.device = env.device
-        try:
-            import torch.distributed as dist
-            if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-                raise RuntimeError("SAC is single-GPU: multi-GPU SAC (a replay per rank and a gradient all-reduce) "
-                                   "is not implemented")
-        except ImportError:
-            pass
+        _refuse_multi_rank("SAC")
         N, D, dev = env.num_envs, env.obs_dim, self.device
         self.n_envs, self.obs_dim = N, D
         torch.manual_seed(cfg.seed)
@@ -214,6 +240,17 @@ class SAC:
         else:
             self.log_ent_coef = None
             self.ent_coef_tensor = torch.tensor(float(cfg.ent_coef), device=dev)
+        self.fused = None
+        if cfg.fused_actor and cuda and D <= 64:
+            self.fused = SacActorB200(self.actor, cfg.action_low, cfg.action_high)
+        self._init_collection(max(1, cfg.buffer_size // N))
+
+    def _init_collection(self, slots, per_agent=()):
+        """Generators, replay ring, staging buffers, statistics, counters and graph slots of the collection loop
+        and the driver, then the first reset: the state that SACPopulation's inherited methods read as well.
+        `per_agent` is the leading shape of the episode and training statistics (() for one agent)."""
+        cfg, env, dev = self.cfg, self.env, self.device
+        N, D = env.num_envs, env.obs_dim
         self.gen_act = torch.Generator(device=dev)
         self.gen_act.manual_seed(cfg.seed + 1)
         self.gen_train = torch.Generator(device=dev)
@@ -222,27 +259,23 @@ class SAC:
         self.high = torch.tensor(cfg.action_high, device=dev)
 
         # replay ring: S slots of N envs
-        S = self.slots = max(1, cfg.buffer_size // N)
+        S = self.slots = slots
         self.rb = dict(obs=torch.zeros((S, N, D), device=dev), next_obs=torch.zeros((S, N, D), device=dev),
                        act=torch.zeros((S, N, 3), device=dev), rew=torch.zeros((S, N), device=dev),
                        done=torch.zeros((S, N), dtype=torch.uint8, device=dev))
         self.pos, self.full = 0, False
         self._pos_t = torch.zeros(1, dtype=torch.long, device=dev)
         self._full_t = torch.zeros(1, dtype=torch.bool, device=dev)
-        self.zero_copy = cuda and hasattr(env, "batch") and not self.use_graphs
+        self.zero_copy = dev.type == "cuda" and hasattr(env, "batch") and not self.use_graphs
         self._trunc = torch.zeros(N, dtype=torch.uint8, device=dev)
         self._env_act = torch.zeros((N, 3), device=dev)
         self._scaled = torch.zeros((N, 3), device=dev)
         self._obs = torch.zeros((N, D), device=dev)
 
-        self.fused = None
-        if cfg.fused_actor and cuda and D <= 64:
-            self.fused = SacActorB200(self.actor, cfg.action_low, cfg.action_high)
-
         self._ep_ret = torch.zeros(N, device=dev)
         self._ep_len = torch.zeros(N, device=dev)
-        self._ep = torch.zeros(4, dtype=torch.float64, device=dev)       # sum return, sum length, successes, episodes
-        self._train_stats = torch.zeros(5, device=dev)                   # critic loss, actor loss, alpha, mean Q, count
+        self._ep = torch.zeros((*per_agent, 4), dtype=torch.float64, device=dev)   # sum return, sum length, successes, episodes
+        self._train_stats = torch.zeros((*per_agent, 5), device=dev)               # critic loss, actor loss, alpha, mean Q, count
         self.num_timesteps = 0
         self.gradient_steps_done = 0
         self._graph_vec = {}

@@ -348,7 +348,12 @@ int salp_lstm_check(void);
  * salp_sac_pack_weights: once per weight update; packed_dev 16-byte aligned.
  * salp_sac_act: obs [N, obs_dim], noise [N, 3] standard normal or NULL, outputs [N, 3]; action_low / high:
  *   host float[3].  Runs on the device that owns packed_dev.
- * salp_sac_check: synchronises the current device; SALP_ERR_CUDA if a kernel gave up on a bounded barrier wait. */
+ * salp_sac_check: synchronises the current device; SALP_ERR_CUDA if a kernel gave up on a bounded barrier wait.
+ * Grouped (K = num_agents actors of one population in one launch, 1 <= K <= 65535): the parameters are stacked
+ *   [K, ...] with the per-agent layout above; packed_dev holds K images of salp_sac_weight_bytes(obs_dim) bytes,
+ *   image k byte-identical to what salp_sac_pack_weights writes for agent k (one launch packs all K).  Rows
+ *   [k n, (k + 1) n) of obs, noise and the outputs belong to agent k (n = envs_per_agent >= 1), and agent k's rows
+ *   are bit-identical to salp_sac_act on image k and those rows.  salp_sac_act / salp_sac_pack_weights are K = 1. */
 int64_t salp_sac_weight_bytes(int32_t obs_dim);
 int salp_sac_pack_weights(const float* w1, const float* b1, const float* w2, const float* b2,
                           const float* w_mu, const float* b_mu, const float* w_log_std, const float* b_log_std,
@@ -356,6 +361,12 @@ int salp_sac_pack_weights(const float* w1, const float* b1, const float* w2, con
 int salp_sac_act(const void* packed_dev, int32_t obs_dim, const float* obs_dev, const float* noise_dev,
                  int64_t n, const float* action_low, const float* action_high,
                  float* env_action_dev, float* scaled_action_dev, void* stream);
+int salp_sac_pack_weights_grouped(const float* w1, const float* b1, const float* w2, const float* b2,
+                                  const float* w_mu, const float* b_mu, const float* w_log_std, const float* b_log_std,
+                                  int32_t num_agents, int32_t obs_dim, void* packed_dev, void* stream);
+int salp_sac_act_grouped(const void* packed_dev, int32_t num_agents, int32_t obs_dim, const float* obs_dev,
+                         const float* noise_dev, int64_t envs_per_agent, const float* action_low,
+                         const float* action_high, float* env_action_dev, float* scaled_action_dev, void* stream);
 int salp_sac_check(void);
 
 /* ---- the element-wise halves of the LEARNER's LSTM step (RecurrentPPO update, BPTT; fp32, any hidden

@@ -3,6 +3,10 @@
 replayed as a CUDA graph) at several env counts; one JSON line per size, first a line with the card.
 
     python tools/bench_sac_act.py [--sizes 8,4096,16384,65536] [--obs-dim 10] [--iters 2000] [--out FILE]
+    python tools/bench_sac_act.py --agents 1,4,16,64 [--sizes 8,1024] ...
+
+With --agents, the grouped kernel instead: salp_sac_act_grouped over K actors of `size` envs each, one
+launch, against K back-to-back salp_sac_act launches on the same rows, one line per (K, size).
 
 Each timing is CUDA events around `iters` back-to-back launches after a warm-up.  FLOP and byte counts
 come from the shapes: 2 N (D 256 + 256 256 + 256 6) flop; obs, noise and both action outputs plus the
@@ -17,7 +21,7 @@ import sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch  # noqa: E402
 
-from grasp_lab_salp_b200.sac import SacActor, SacActorB200  # noqa: E402
+from grasp_lab_salp_b200.sac import SacActor, SacActorB200, SacActorGroupB200  # noqa: E402
 
 
 def card():
@@ -45,6 +49,7 @@ def main():
     ap.add_argument("--obs-dim", type=int, default=10)
     ap.add_argument("--iters", type=int, default=2000)
     ap.add_argument("--out", default=None)
+    ap.add_argument("--agents", default=None, help="comma-separated population sizes: time salp_sac_act_grouped")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("bench_sac_act.py needs a CUDA device")
@@ -59,6 +64,8 @@ def main():
     emit(card())
     torch.manual_seed(0)
     D = args.obs_dim
+    if args.agents:
+        return bench_grouped(args, emit)
     actor = SacActor(D).cuda()
     lo, hi = torch.tensor([0.0, 0.0, -1.0], device="cuda"), torch.tensor([1.0, 1.0, 1.0], device="cuda")
     fused = SacActorB200(actor, lo.tolist(), hi.tolist())
@@ -89,6 +96,31 @@ def main():
                   torch_graph_us=round(t_g, 2), kernel_tflops=round(flop / t_k * 1e-6, 2),
                   kernel_gbytes_per_s=round(nbytes / t_k * 1e-3, 1), torch_graph_tflops=round(flop / t_g * 1e-6, 2),
                   speedup_vs_graph=round(t_g / t_k, 2)))
+
+
+def bench_grouped(args, emit):
+    D = args.obs_dim
+    lo, hi = [0.0, 0.0, -1.0], [1.0, 1.0, 1.0]
+    for K in [int(k) for k in args.agents.split(",")]:
+        actors = [SacActor(D).cuda() for _ in range(K)]
+        group = SacActorGroupB200([torch.stack([p.detach() for p in ps]).contiguous()
+                                   for ps in zip(*(a.parameters() for a in actors))], lo, hi)
+        singles = [SacActorB200(a, lo, hi) for a in actors]
+        for n in [int(s) for s in args.sizes.split(",")]:
+            obs = torch.randn(K * n, D, device="cuda")
+            noise = torch.randn(K * n, 3, device="cuda")
+            env_a, a = torch.empty(K * n, 3, device="cuda"), torch.empty(K * n, 3, device="cuda")
+            rows = [(obs[k * n:(k + 1) * n], noise[k * n:(k + 1) * n], env_a[k * n:(k + 1) * n], a[k * n:(k + 1) * n])
+                    for k in range(K)]
+
+            def one_by_one():
+                for s, r in zip(singles, rows):
+                    s.act(*r)
+            t_g = time_it(lambda: group.act(obs, noise, env_a, a), args.iters)
+            t_s = time_it(one_by_one, max(1, args.iters // K))
+            group.check()
+            emit(dict(agents=K, envs_per_agent=n, obs_dim=D, grouped_us=round(t_g, 2), k_single_launches_us=round(t_s, 2),
+                      speedup=round(t_s / t_g, 2), grouped_us_per_agent=round(t_g / K, 2)))
 
 
 if __name__ == "__main__":
