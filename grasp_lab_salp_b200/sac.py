@@ -37,6 +37,12 @@ With ``cuda_graphs=True`` one vec step and one gradient step are each replayed a
 vec-step graph fills the ring through staging buffers (index_copy_ at a device-side position), since
 a captured graph cannot follow a moving slot pointer.
 
+Everything that does not depend on how the learner stores its weights -- the config checks, collection,
+replay sampling, ``learn``, its log rows and ``evaluate`` -- is ``_SACDriver``, written for K agents side by
+side and shared with ``sac_population.SACPopulation``.  ``SAC`` is its K = 1 case: it adds the nn.Modules,
+torch.optim.Adam, the SB3 gradient step (``train_step``) and save / load, and returns agent 0 of the shared
+per-agent sample, log rows and evaluation.
+
 The learner runs on CPU too, through ``ppo.HostEnv``.  Multi-GPU SAC is not implemented: under an
 initialised torch.distributed with more than one rank the constructor refuses.
 """
@@ -45,7 +51,7 @@ from __future__ import annotations
 import ctypes as C
 import math
 import time
-from dataclasses import dataclass
+from dataclasses import dataclass, fields
 
 import torch
 import torch.nn as nn
@@ -78,9 +84,24 @@ class SACConfig:
     action_high: tuple = (1.0, 1.0, 1.0)
 
 
+PER_AGENT = ("seed", "learning_rate", "gamma", "tau", "target_entropy", "ent_coef")   # may differ in a population
+
+
 # ------------------------------------------------------------------------------------------------
 # networks (SB3 SACPolicy, net_arch [256, 256])
 # ------------------------------------------------------------------------------------------------
+def squashed_gaussian(mean, log_std, eps):
+    """Reparametrised squashed-Gaussian sample with standard-normal `eps` [..., 3] and its log-prob summed over
+    the last dimension, written out exactly as torch.distributions.Normal and SB3's
+    SquashedDiagGaussianDistribution compute them."""
+    std = torch.ones_like(mean) * log_std.exp()
+    u = mean + eps * std
+    a = torch.tanh(u)
+    logp = (-((u - mean) ** 2) / (2 * std ** 2) - std.log() - math.log(math.sqrt(2 * math.pi))).sum(dim=-1)
+    logp = logp - torch.sum(torch.log(1 - a ** 2 + 1e-6), dim=-1)
+    return a, logp
+
+
 class SacActor(nn.Module):
     def __init__(self, obs_dim, act_dim=ACT_DIM, hidden=HIDDEN):
         super().__init__()
@@ -94,16 +115,8 @@ class SacActor(nn.Module):
         return self.mu(latent), torch.clamp(self.log_std(latent), LOG_STD_MIN, LOG_STD_MAX)
 
     def action_log_prob(self, obs, eps):
-        """Reparametrised squashed-Gaussian sample with standard-normal `eps` [B, 3] and its log-prob,
-        written out exactly as torch.distributions.Normal and SB3's SquashedDiagGaussianDistribution
-        compute them."""
-        mean, log_std = self(obs)
-        std = torch.ones_like(mean) * log_std.exp()
-        u = mean + eps * std
-        a = torch.tanh(u)
-        logp = (-((u - mean) ** 2) / (2 * std ** 2) - std.log() - math.log(math.sqrt(2 * math.pi))).sum(dim=1)
-        logp = logp - torch.sum(torch.log(1 - a ** 2 + 1e-6), dim=1)
-        return a, logp
+        """squashed_gaussian of this actor on obs [B, D]: actions [B, 3], log-prob [B]."""
+        return squashed_gaussian(*self(obs), eps)
 
 
 class SacCritic(nn.Module):
@@ -212,45 +225,46 @@ def _refuse_multi_rank(name):
         pass
 
 
-class SAC:
-    def __init__(self, env, config: SACConfig | None = None):
-        self.env = env
-        self.cfg = cfg = config or SACConfig()
-        self.device = env.device
-        _refuse_multi_rank("SAC")
-        N, D, dev = env.num_envs, env.obs_dim, self.device
-        self.n_envs, self.obs_dim = N, D
-        torch.manual_seed(cfg.seed)
-        self.actor = SacActor(D).to(dev)
-        self.critic = SacCritic(D).to(dev)
-        self.critic_target = SacCritic(D).to(dev)
-        self.critic_target.load_state_dict(self.critic.state_dict())
-        self.critic_target.requires_grad_(False)
-        cuda = dev.type == "cuda"
-        self.use_graphs = bool(cfg.cuda_graphs) and cuda
-        adam = dict(lr=cfg.learning_rate, capturable=cuda)
-        self.actor_opt = torch.optim.Adam(self.actor.parameters(), **adam)
-        self.critic_opt = torch.optim.Adam(self.critic.parameters(), **adam)
-        self.auto_ent = isinstance(cfg.ent_coef, str)
-        if self.auto_ent:
-            if cfg.ent_coef != "auto":
-                raise ValueError("ent_coef must be 'auto' or a float")
-            self.log_ent_coef = torch.log(torch.ones(1, device=dev)).requires_grad_(True)
-            self.ent_opt = torch.optim.Adam([self.log_ent_coef], **adam)
-        else:
-            self.log_ent_coef = None
-            self.ent_coef_tensor = torch.tensor(float(cfg.ent_coef), device=dev)
-        self.fused = None
-        if cfg.fused_actor and cuda and D <= 64:
-            self.fused = SacActorB200(self.actor, cfg.action_low, cfg.action_high)
-        self._init_collection(max(1, cfg.buffer_size // N))
+class _SACDriver:
+    """Everything of SAC that does not depend on how the learner stores its weights, for K = len(configs) agents on
+    one env of K n envs, agent k on env rows [k n, (k + 1) n) (SAC is K = 1): the config checks, collection into
+    one slot-major replay ring, per-agent sampling, ``learn``, its log rows and ``evaluate``.
 
-    def _init_collection(self, slots, per_agent=()):
+    A learner calls ``__init__``, builds its networks, sets ``fused`` (a SacActorGroupB200 or None) and
+    ``actor_opt`` / ``critic_opt`` / ``ent_opt``, then calls ``_init_collection``.  It supplies
+    ``_policy_forward(obs)``, the torch actor on obs [K m, D] giving (mu, clamped log_std) [K m, 3] with agent k
+    on rows [k m, (k + 1) m), and ``train_step()``, one gradient step of every agent on ``sample``'s batch."""
+
+    def __init__(self, env, configs):
+        configs = list(configs)
+        K = len(configs)
+        if K < 1:
+            raise ValueError("a population needs at least one config")
+        c0 = configs[0]
+        for f in fields(SACConfig):
+            if f.name not in PER_AGENT and any(getattr(c, f.name) != getattr(c0, f.name) for c in configs):
+                raise ValueError(f"SACConfig.{f.name} must be equal across the population (only "
+                                 f"{', '.join(PER_AGENT)} may differ per agent)")
+        auto = [isinstance(c.ent_coef, str) for c in configs]
+        if any(auto) and not (all(auto) and all(c.ent_coef == "auto" for c in configs)):
+            raise ValueError("ent_coef must be 'auto' for every agent or a float for every agent")
+        if env.num_envs % K:
+            raise ValueError(f"env.num_envs ({env.num_envs}) must be a multiple of the population size ({K})")
+        _refuse_multi_rank(type(self).__name__)
+        self.env, self.configs = env, configs
+        self.cfg = c0                             # (read for the fields shared by every agent)
+        self.device = env.device
+        N = env.num_envs
+        self.num_agents, self.n_total, self.n_envs, self.obs_dim = K, N, N // K, env.obs_dim
+        self.use_graphs = bool(c0.cuda_graphs) and self.device.type == "cuda"
+        self.auto_ent = all(auto)
+
+    def _init_collection(self):
         """Generators, replay ring, staging buffers, statistics, counters and graph slots of the collection loop
-        and the driver, then the first reset: the state that SACPopulation's inherited methods read as well.
-        `per_agent` is the leading shape of the episode and training statistics (() for one agent)."""
+        and the driver, then the first reset.  The ring has buffer_size // n slots of K n envs (agent k's ring is
+        its n columns); the generators are seeded from the first config."""
         cfg, env, dev = self.cfg, self.env, self.device
-        N, D = env.num_envs, env.obs_dim
+        K, N, D = self.num_agents, self.n_total, self.obs_dim
         self.gen_act = torch.Generator(device=dev)
         self.gen_act.manual_seed(cfg.seed + 1)
         self.gen_train = torch.Generator(device=dev)
@@ -259,7 +273,7 @@ class SAC:
         self.high = torch.tensor(cfg.action_high, device=dev)
 
         # replay ring: S slots of N envs
-        S = self.slots = slots
+        S = self.slots = max(1, cfg.buffer_size // self.n_envs)
         self.rb = dict(obs=torch.zeros((S, N, D), device=dev), next_obs=torch.zeros((S, N, D), device=dev),
                        act=torch.zeros((S, N, 3), device=dev), rew=torch.zeros((S, N), device=dev),
                        done=torch.zeros((S, N), dtype=torch.uint8, device=dev))
@@ -274,8 +288,8 @@ class SAC:
 
         self._ep_ret = torch.zeros(N, device=dev)
         self._ep_len = torch.zeros(N, device=dev)
-        self._ep = torch.zeros((*per_agent, 4), dtype=torch.float64, device=dev)   # sum return, sum length, successes, episodes
-        self._train_stats = torch.zeros((*per_agent, 5), device=dev)               # critic loss, actor loss, alpha, mean Q, count
+        self._ep = torch.zeros((K, 4), dtype=torch.float64, device=dev)   # sum return, sum length, successes, episodes
+        self._train_stats = torch.zeros((K, 5), device=dev)               # critic loss, actor loss, alpha, mean Q, count
         self.num_timesteps = 0
         self.gradient_steps_done = 0
         self._graph_vec = {}
@@ -289,13 +303,14 @@ class SAC:
 
     # ---- acting ----
     def _policy_act(self, obs, env_out, scaled_out, deterministic=False, generator=None):
-        """Actor forward into env_out / scaled_out (fused kernel or torch)."""
+        """Actor forward of agent k on rows [k m, (k + 1) m) of obs [K m, D] into env_out / scaled_out (fused
+        kernel or torch)."""
         noise = None if deterministic else torch.randn((obs.shape[0], 3), device=self.device, generator=generator)
         if self.fused is not None:
             self.fused.act(obs, noise, env_out, scaled_out)
             return
         with torch.no_grad():
-            mean, log_std = self.actor(obs)
+            mean, log_std = self._policy_forward(obs)
             u = mean if noise is None else mean + noise * log_std.exp()
             a = torch.tanh(u)
             scaled_out.copy_(a)
@@ -303,14 +318,14 @@ class SAC:
 
     def _random_act(self, env_out, scaled_out):
         """SB3 warm-up: action_space.sample() (uniform on the Box), stored as scale_action() of it."""
-        u = torch.rand((self.n_envs, 3), device=self.device, generator=self.gen_act)
+        u = torch.rand((self.n_total, 3), device=self.device, generator=self.gen_act)
         a_env = self.low + u * (self.high - self.low)
         env_out.copy_(a_env)
         scaled_out.copy_(2.0 * ((a_env - self.low) / (self.high - self.low)) - 1.0)
 
     @torch.no_grad()
     def predict(self, obs, deterministic=True):
-        """Env-space actions [n, 3] for obs [n, D] (SB3 predict)."""
+        """Env-space actions [n, 3] for obs [n, D] (SB3 predict); agent k acts on rows [k m, (k + 1) m)."""
         obs = obs.to(self.device, torch.float32).contiguous()
         env_out = torch.empty((obs.shape[0], 3), device=self.device)
         scaled = torch.empty_like(env_out)
@@ -318,17 +333,22 @@ class SAC:
         return env_out
 
     # ---- collection ----
-    def _bookkeep(self, rew, term, trunc):
-        raw = torch.nan_to_num(rew, nan=0.0, posinf=0.0, neginf=0.0)
+    def _clip_reward(self, rew):
+        """The learner-side reward clip: non-finite rewards count as 0, then |r| <= reward_clip (0 disables it)."""
+        rew = torch.nan_to_num(rew, nan=0.0, posinf=0.0, neginf=0.0)
         if self.cfg.reward_clip > 0:
-            raw = raw.clamp(-self.cfg.reward_clip, self.cfg.reward_clip)
+            rew = rew.clamp(-self.cfg.reward_clip, self.cfg.reward_clip)
+        return rew
+
+    def _bookkeep(self, rew, term, trunc):
+        raw = self._clip_reward(rew)
         term, trunc = term.bool(), trunc.bool()
         done = term | trunc
         self._ep_ret += raw
         self._ep_len += 1
         d = done.to(torch.float64)
-        self._ep += torch.stack([(self._ep_ret.double() * d).sum(), (self._ep_len.double() * d).sum(),
-                                 (term.double() * d).sum(), d.sum()])
+        per_env = torch.stack([self._ep_ret.double() * d, self._ep_len.double() * d, term.double() * d, d], dim=1)
+        self._ep += per_env.view(self.num_agents, -1, 4).sum(1)
         keep = (~done).float()
         self._ep_ret *= keep
         self._ep_len *= keep
@@ -385,75 +405,24 @@ class SAC:
 
     # ---- learning ----
     def sample(self, batch_size):
-        """Uniform over (slot, env) among the complete slots; once the ring has wrapped the slot being
-        filled is skipped.  Device-side (capturable): the fill level lives in device tensors."""
-        S, N, dev, g = self.slots, self.n_envs, self.device, self.gen_train
+        """`batch_size` transitions per agent ([K, B, ...]): uniform over (slot, env of that agent) among the
+        complete slots; once the ring has wrapped the slot being filled is skipped.  Device-side (capturable): the
+        fill level lives in device tensors."""
+        S, N, n, K, dev, g = self.slots, self.n_total, self.n_envs, self.num_agents, self.device, self.gen_train
         pos, full = self._pos_t, self._full_t
         count = torch.where(full, torch.full_like(pos, S - 1), pos)
         start = torch.where(full, pos + 1, torch.zeros_like(pos))
-        u = torch.rand(batch_size, device=dev, generator=g, dtype=torch.float64)
-        k = torch.minimum((u * count).long(), count - 1)
-        slot = (start + k) % S
-        env = torch.minimum((torch.rand(batch_size, device=dev, generator=g, dtype=torch.float64) * N).long(),
-                            torch.full_like(slot, N - 1))
+        u = torch.rand((K, batch_size), device=dev, generator=g, dtype=torch.float64)
+        slot = (start + torch.minimum((u * count).long(), count - 1)) % S
+        env = torch.minimum((torch.rand((K, batch_size), device=dev, generator=g, dtype=torch.float64) * n).long(),
+                            torch.full_like(slot, n - 1))
+        env = env + torch.arange(K, device=dev).unsqueeze(1) * n
         idx = slot * N + env
         rb = self.rb
-        rew = torch.nan_to_num(rb["rew"].view(-1)[idx], nan=0.0, posinf=0.0, neginf=0.0)
-        if self.cfg.reward_clip > 0:
-            rew = rew.clamp(-self.cfg.reward_clip, self.cfg.reward_clip)
+        rew = self._clip_reward(rb["rew"].view(-1)[idx])
         return dict(obs=rb["obs"].view(S * N, -1)[idx], actions=rb["act"].view(S * N, -1)[idx],
-                    next_obs=rb["next_obs"].view(S * N, -1)[idx], rewards=rew.unsqueeze(1),
-                    dones=rb["done"].view(-1)[idx].float().unsqueeze(1), slot=slot, env=env)
-
-    def train_step(self, batch=None, eps=None):
-        """One SB3 gradient step.  `batch` (dict of obs, actions, next_obs, rewards [B, 1], dones [B, 1])
-        and `eps` (standard-normal noise of the two actor samples) are drawn here unless given."""
-        cfg = self.cfg
-        if batch is None:
-            batch = self.sample(cfg.batch_size)
-        B = batch["obs"].shape[0]
-        if eps is None:
-            eps = (torch.randn((B, 3), device=self.device, generator=self.gen_train),
-                   torch.randn((B, 3), device=self.device, generator=self.gen_train))
-        actions_pi, log_prob = self.actor.action_log_prob(batch["obs"], eps[0])
-        log_prob = log_prob.reshape(-1, 1)
-        if self.auto_ent:
-            ent_coef = torch.exp(self.log_ent_coef.detach())
-            ent_coef_loss = -(self.log_ent_coef * (log_prob + cfg.target_entropy).detach()).mean()
-            self.ent_opt.zero_grad()
-            ent_coef_loss.backward()
-            self.ent_opt.step()
-        else:
-            ent_coef = self.ent_coef_tensor
-        with torch.no_grad():
-            next_actions, next_log_prob = self.actor.action_log_prob(batch["next_obs"], eps[1])
-            next_q_values = torch.cat(self.critic_target(batch["next_obs"], next_actions), dim=1)
-            next_q_values, _ = torch.min(next_q_values, dim=1, keepdim=True)
-            next_q_values = next_q_values - ent_coef * next_log_prob.reshape(-1, 1)
-            target_q_values = batch["rewards"] + (1 - batch["dones"]) * cfg.gamma * next_q_values
-        current_q_values = self.critic(batch["obs"], batch["actions"])
-        critic_loss = 0.5 * sum(F.mse_loss(current_q, target_q_values) for current_q in current_q_values)
-        self.critic_opt.zero_grad()
-        critic_loss.backward()
-        self.critic_opt.step()
-        q_values_pi = torch.cat(self.critic(batch["obs"], actions_pi), dim=1)
-        min_qf_pi, _ = torch.min(q_values_pi, dim=1, keepdim=True)
-        actor_loss = (ent_coef * log_prob - min_qf_pi).mean()
-        self.actor_opt.zero_grad()
-        actor_loss.backward()
-        self.actor_opt.step()
-        self._train_calls += 1
-        if (self._train_calls - 1) % cfg.target_update_interval == 0:
-            with torch.no_grad():
-                tp, sp = list(self.critic_target.parameters()), list(self.critic.parameters())
-                torch._foreach_mul_(tp, 1 - cfg.tau)
-                torch._foreach_add_(tp, sp, alpha=cfg.tau)
-        with torch.no_grad():
-            mean_q = torch.stack([q.mean() for q in current_q_values]).mean()
-            self._train_stats += torch.stack([critic_loss.detach(), actor_loss.detach(), ent_coef.reshape(()),
-                                              mean_q, torch.ones((), device=self.device)])
-        return dict(critic_loss=critic_loss, actor_loss=actor_loss, ent_coef=ent_coef,
-                    ent_coef_loss=ent_coef_loss if self.auto_ent else None)
+                    next_obs=rb["next_obs"].view(S * N, -1)[idx], rewards=rew.unsqueeze(-1),
+                    dones=rb["done"].view(-1)[idx].float().unsqueeze(-1), slot=slot, env=env)
 
     def _train(self):
         for _ in range(self.cfg.gradient_steps):
@@ -505,7 +474,10 @@ class SAC:
                 ev = self.evaluate(eval_env, n_eval_episodes)
                 next_eval += eval_every
             if self.num_timesteps >= next_log or self.num_timesteps >= total_timesteps:
-                row = self._row(collect_s, train_s, ev)
+                row = self._row(collect_s, train_s)
+                if ev:
+                    row.update(eval_return=ev["mean_return"], eval_success=ev["success_rate"],
+                               eval_length=ev["mean_length"])
                 history.append(row)
                 if log:
                     log(row)
@@ -514,48 +486,146 @@ class SAC:
                 ev = {}
         return history
 
-    def _row(self, collect_s, train_s, ev):
-        ep = self._ep.tolist()
-        ts = self._train_stats.tolist()
+    def _row(self, collect_s, train_s):
+        """The training and episode statistics since the last row (per agent: lists of K), which it zeroes."""
+        ep, ts = self._ep.tolist(), self._train_stats.tolist()
         self._ep.zero_()
         self._train_stats.zero_()
-        ne, nt = int(ep[3]), ts[4]
         nan = float("nan")
-        row = dict(env_steps=self.num_timesteps, gradient_steps=self.gradient_steps_done,
-                   ent_coef=ts[2] / nt if nt else nan, critic_loss=ts[0] / nt if nt else nan,
-                   actor_loss=ts[1] / nt if nt else nan, mean_q=ts[3] / nt if nt else nan, episodes=ne,
-                   mean_episode_return=ep[0] / ne if ne else nan, mean_episode_length=ep[1] / ne if ne else nan,
-                   success_rate=ep[2] / ne if ne else nan, collect_seconds=collect_s, train_seconds=train_s)
-        if ev:
-            row.update(eval_return=ev["mean_return"], eval_success=ev["success_rate"], eval_length=ev["mean_length"])
-        return row
+
+        def ratio(rows, i, j):
+            return [r[i] / r[j] if r[j] else nan for r in rows]
+        return dict(env_steps=self.num_timesteps, gradient_steps=self.gradient_steps_done,
+                    ent_coef=ratio(ts, 2, 4), critic_loss=ratio(ts, 0, 4), actor_loss=ratio(ts, 1, 4),
+                    mean_q=ratio(ts, 3, 4), episodes=[int(e[3]) for e in ep], mean_episode_return=ratio(ep, 0, 3),
+                    mean_episode_length=ratio(ep, 1, 3), success_rate=ratio(ep, 2, 3), collect_seconds=collect_s,
+                    train_seconds=train_s)
 
     @torch.no_grad()
     def evaluate(self, env, n_episodes=10):
-        """Deterministic episodes on a separate env (SB3 EvalCallback(deterministic=True) via
-        evaluate_policy: env i contributes (n_episodes + i) // n_envs episodes)."""
-        n = env.num_envs
-        targets = torch.tensor([(n_episodes + i) // n for i in range(n)])
-        counts = torch.zeros(n, dtype=torch.long)
-        rets, lens, succ = [], [], []
-        cur_r, cur_l = torch.zeros(n, dtype=torch.float64), torch.zeros(n, dtype=torch.long)
+        """Deterministic episodes (SB3 EvalCallback(deterministic=True) via evaluate_policy) on an eval env of
+        K m envs, agent k acting on rows [k m, (k + 1) m): env i of a slice contributes (n_episodes + i) // m
+        episodes.  Per-agent lists of mean_return, mean_length, success_rate and episodes.  The quotas are read
+        back every 16 steps, so the env may step up to 15 times past the last recorded episode."""
+        K, N = self.num_agents, env.num_envs
+        if N % K:
+            raise ValueError(f"the eval env's num_envs ({N}) must be a multiple of the population size ({K})")
+        m, dev = N // K, env.device
+        targets = ((n_episodes + torch.arange(m, device=dev)) // m).repeat(K)
+        counts = torch.zeros(N, dtype=torch.long, device=dev)
+        sums = torch.zeros((K, 4), dtype=torch.float64, device=dev)        # return, length, successes, episodes
+        cur_r = torch.zeros(N, dtype=torch.float64, device=dev)
+        cur_l = torch.zeros(N, dtype=torch.float64, device=dev)
         obs = env.reset_t()
-        while bool((counts < targets).any()):
+        step = 0
+        while step % 16 or bool((counts < targets).any()):                # (a finished env records nothing more)
             a = self.predict(obs.float(), deterministic=True)
             obs, rew, term, trunc, _ = env.step_t(a)
-            r = torch.nan_to_num(rew, nan=0.0, posinf=0.0, neginf=0.0).double().cpu()
-            t, d = term.bool().cpu(), (term.bool() | trunc.bool()).cpu()
-            cur_r += r
+            t = term.bool()
+            d = t | trunc.bool()
+            cur_r += torch.nan_to_num(rew, nan=0.0, posinf=0.0, neginf=0.0).double()
             cur_l += 1
-            for i in torch.nonzero(d & (counts < targets)).flatten().tolist():
-                rets.append(cur_r[i].item())
-                lens.append(cur_l[i].item())
-                succ.append(float(t[i]))
-                counts[i] += 1
-            cur_r[d] = 0.0
-            cur_l[d] = 0
-        k = len(rets)
-        return dict(mean_return=sum(rets) / k, mean_length=sum(lens) / k, success_rate=sum(succ) / k, episodes=k)
+            rec = d & (counts < targets)
+            w = rec.double()
+            sums += torch.stack([cur_r * w, cur_l * w, t.double() * w, w], dim=1).view(K, m, 4).sum(1)
+            counts += rec.long()
+            cur_r.masked_fill_(d, 0.0)
+            cur_l.masked_fill_(d, 0.0)
+            step += 1
+        s = sums.tolist()
+        return dict(mean_return=[x[0] / x[3] for x in s], mean_length=[x[1] / x[3] for x in s],
+                    success_rate=[x[2] / x[3] for x in s], episodes=[int(x[3]) for x in s])
+
+
+class SAC(_SACDriver):
+    def __init__(self, env, config: SACConfig | None = None):
+        super().__init__(env, [config or SACConfig()])
+        cfg, dev, D = self.cfg, self.device, self.obs_dim
+        torch.manual_seed(cfg.seed)
+        self.actor = SacActor(D).to(dev)
+        self.critic = SacCritic(D).to(dev)
+        self.critic_target = SacCritic(D).to(dev)
+        self.critic_target.load_state_dict(self.critic.state_dict())
+        self.critic_target.requires_grad_(False)
+        cuda = dev.type == "cuda"
+        adam = dict(lr=cfg.learning_rate, capturable=cuda)
+        self.actor_opt = torch.optim.Adam(self.actor.parameters(), **adam)
+        self.critic_opt = torch.optim.Adam(self.critic.parameters(), **adam)
+        if self.auto_ent:
+            self.log_ent_coef = torch.log(torch.ones(1, device=dev)).requires_grad_(True)
+            self.ent_opt = torch.optim.Adam([self.log_ent_coef], **adam)
+        else:
+            self.log_ent_coef = None
+            self.ent_coef_tensor = torch.tensor(float(cfg.ent_coef), device=dev)
+        self.fused = None
+        if cfg.fused_actor and cuda and D <= 64:
+            self.fused = SacActorB200(self.actor, cfg.action_low, cfg.action_high)
+        self._init_collection()
+
+    def _policy_forward(self, obs):
+        return self.actor(obs)
+
+    def sample(self, batch_size):
+        """`batch_size` transitions [B, ...], uniform over (slot, env) among the complete slots; once the ring has
+        wrapped the slot being filled is skipped.  Device-side (capturable)."""
+        return {k: v[0] for k, v in super().sample(batch_size).items()}
+
+    def train_step(self, batch=None, eps=None):
+        """One SB3 gradient step.  `batch` (dict of obs, actions, next_obs, rewards [B, 1], dones [B, 1])
+        and `eps` (standard-normal noise of the two actor samples) are drawn here unless given."""
+        cfg = self.cfg
+        if batch is None:
+            batch = self.sample(cfg.batch_size)
+        B = batch["obs"].shape[0]
+        if eps is None:
+            eps = (torch.randn((B, 3), device=self.device, generator=self.gen_train),
+                   torch.randn((B, 3), device=self.device, generator=self.gen_train))
+        actions_pi, log_prob = self.actor.action_log_prob(batch["obs"], eps[0])
+        log_prob = log_prob.reshape(-1, 1)
+        if self.auto_ent:
+            ent_coef = torch.exp(self.log_ent_coef.detach())
+            ent_coef_loss = -(self.log_ent_coef * (log_prob + cfg.target_entropy).detach()).mean()
+            self.ent_opt.zero_grad()
+            ent_coef_loss.backward()
+            self.ent_opt.step()
+        else:
+            ent_coef = self.ent_coef_tensor
+        with torch.no_grad():
+            next_actions, next_log_prob = self.actor.action_log_prob(batch["next_obs"], eps[1])
+            next_q_values = torch.cat(self.critic_target(batch["next_obs"], next_actions), dim=1)
+            next_q_values, _ = torch.min(next_q_values, dim=1, keepdim=True)
+            next_q_values = next_q_values - ent_coef * next_log_prob.reshape(-1, 1)
+            target_q_values = batch["rewards"] + (1 - batch["dones"]) * cfg.gamma * next_q_values
+        current_q_values = self.critic(batch["obs"], batch["actions"])
+        critic_loss = 0.5 * sum(F.mse_loss(current_q, target_q_values) for current_q in current_q_values)
+        self.critic_opt.zero_grad()
+        critic_loss.backward()
+        self.critic_opt.step()
+        q_values_pi = torch.cat(self.critic(batch["obs"], actions_pi), dim=1)
+        min_qf_pi, _ = torch.min(q_values_pi, dim=1, keepdim=True)
+        actor_loss = (ent_coef * log_prob - min_qf_pi).mean()
+        self.actor_opt.zero_grad()
+        actor_loss.backward()
+        self.actor_opt.step()
+        self._train_calls += 1
+        if (self._train_calls - 1) % cfg.target_update_interval == 0:
+            with torch.no_grad():
+                tp, sp = list(self.critic_target.parameters()), list(self.critic.parameters())
+                torch._foreach_mul_(tp, 1 - cfg.tau)
+                torch._foreach_add_(tp, sp, alpha=cfg.tau)
+        with torch.no_grad():
+            mean_q = torch.stack([q.mean() for q in current_q_values]).mean()
+            self._train_stats += torch.stack([critic_loss.detach(), actor_loss.detach(), ent_coef.reshape(()),
+                                              mean_q, torch.ones((), device=self.device)])
+        return dict(critic_loss=critic_loss, actor_loss=actor_loss, ent_coef=ent_coef,
+                    ent_coef_loss=ent_coef_loss if self.auto_ent else None)
+
+    def _row(self, collect_s, train_s):
+        return {k: v[0] if isinstance(v, list) else v for k, v in super()._row(collect_s, train_s).items()}
+
+    def evaluate(self, env, n_episodes=10):
+        """The shared evaluation with scalar results: env i contributes (n_episodes + i) // n_envs episodes."""
+        return {k: v[0] for k, v in super().evaluate(env, n_episodes).items()}
 
     # ---- persistence ----
     def save(self, path):

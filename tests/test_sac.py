@@ -1,8 +1,9 @@
 """SAC on the batched simulator (grasp_lab_salp_b200/sac.py) and its rollout-side actor kernel
 (csrc/salp_sac.cu).  CPU: one gradient step against a line-by-line restatement of stable-baselines3's
-SAC.train(), the squashed-Gaussian log-prob, replay semantics on a wrapping ring, the same curve on the
-host build of the kernel body and on the C oracle, argument checks, save / load.  GPU: salp_sac_act
-against float64 and fp32 torch actors, rollout / ring / CUDA-graph equivalence, learning."""
+SAC.train(), the squashed-Gaussian log-prob, replay semantics on a wrapping ring, evaluation against a
+restatement of SB3's evaluate_policy quotas, the same curve on the host build of the kernel body and on the C
+oracle, argument checks, save / load.  GPU: salp_sac_act against float64 and fp32 torch actors, rollout / ring /
+CUDA-graph equivalence, learning."""
 import copy
 import ctypes as C
 import math
@@ -119,6 +120,50 @@ def _sb3_train_step(actor, critic, critic_target, log_ent_coef, ent_coef_tensor,
             target_param.data.mul_(1 - tau)
             torch.add(target_param.data, param.data, alpha=tau, out=target_param.data)
     return critic_loss, actor_loss, ent_coef_loss
+
+
+def _sb3_evaluate(predict, env, n_episodes, agents=1):
+    """stable-baselines3 evaluate_policy(deterministic=True) restated as a host loop over the env's K = `agents`
+    slices of m envs: env i of a slice contributes (n_episodes + i) // m episodes to its agent.  Per-agent list of
+    dicts of mean_return, mean_length, success_rate and episodes."""
+    n = env.num_envs
+    m = n // agents
+    targets = torch.tensor([(n_episodes + i % m) // m for i in range(n)])
+    counts = torch.zeros(n, dtype=torch.long)
+    rets, lens, succ = ([[] for _ in range(agents)] for _ in range(3))
+    cur_r, cur_l = torch.zeros(n, dtype=torch.float64), torch.zeros(n, dtype=torch.long)
+    obs = env.reset_t()
+    while bool((counts < targets).any()):
+        a = predict(obs.float(), deterministic=True)
+        obs, rew, term, trunc, _ = env.step_t(a)
+        r = torch.nan_to_num(rew, nan=0.0, posinf=0.0, neginf=0.0).double().cpu()
+        t, d = term.bool().cpu(), (term.bool() | trunc.bool()).cpu()
+        cur_r += r
+        cur_l += 1
+        for i in torch.nonzero(d & (counts < targets)).flatten().tolist():
+            rets[i // m].append(cur_r[i].item())
+            lens[i // m].append(cur_l[i].item())
+            succ[i // m].append(float(t[i]))
+            counts[i] += 1
+        cur_r[d] = 0.0
+        cur_l[d] = 0
+    return [dict(mean_return=sum(r) / len(r), mean_length=sum(ln) / len(r), success_rate=sum(s) / len(r),
+                 episodes=len(r)) for r, ln, s in zip(rets, lens, succ)]
+
+
+def _assert_eval_matches(mine, ref):
+    """Episode counts, lengths and success rates exactly, returns to 1e-12 relative."""
+    for key in ("episodes", "mean_length", "success_rate"):
+        assert mine[key] == ref[key], key
+    assert mine["mean_return"] == pytest.approx(ref["mean_return"], rel=1e-12, abs=0)
+
+
+def test_evaluate_matches_sb3_quota_restatement():
+    sac = SAC(_host_env(4), SACConfig(seed=3))
+    ref = _sb3_evaluate(sac.predict, _host_env(3, seed=9), 5)[0]     # quotas 1, 2, 2
+    ev = sac.evaluate(_host_env(3, seed=9), 5)
+    assert ev["episodes"] == 5
+    _assert_eval_matches(ev, ref)
 
 
 @pytest.mark.parametrize("ent_coef", ["auto", 0.2])

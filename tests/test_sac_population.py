@@ -1,7 +1,8 @@
 """A population of SAC agents trained side by side (grasp_lab_salp_b200/sac_population.py) and the grouped
 rollout actor kernel (salp_sac_act_grouped, csrc/salp_sac.cu).  CPU: initialisation, per-agent gradient steps
-against the stable-baselines3 restatement of test_sac.py, per-agent replay, a short learn() on the host
-build of the kernel body, argument checks, save_agent.  GPU: the grouped kernel against salp_sac_act, a
+against the stable-baselines3 restatement of test_sac.py, per-agent replay, one agent collecting as SAC does,
+per-agent evaluation against test_sac.py's evaluate_policy restatement, a short learn() on the host build of
+the kernel body, argument checks, save_agent.  GPU: the grouped kernel against salp_sac_act, a
 K n-env batch against K separate batches, CUDA-graph equivalence, learning."""
 import ctypes as C
 import time
@@ -12,7 +13,7 @@ import torch
 from grasp_lab_salp_b200 import _lib
 from grasp_lab_salp_b200.sac import SAC, SacActor, SacActorB200, SacActorGroupB200, SACConfig, SacCritic
 from grasp_lab_salp_b200.sac_population import SACPopulation
-from test_sac import _host_env, _sb3_train_step, _TaggedEnv
+from test_sac import _assert_eval_matches, _host_env, _sb3_evaluate, _sb3_train_step, _TaggedEnv
 
 
 def _agent_modules(pop, k):
@@ -112,6 +113,31 @@ def test_replay_is_per_agent_on_a_wrapping_ring():
         assert torch.equal(s["next_obs"][k, :, 0], tags)
     t_obs, t_next = s["obs"][..., 1], s["next_obs"][..., 1]
     assert ((t_obs == t_next - 1) | (t_obs == -1)).all()
+
+
+def test_one_agent_collects_like_sac():
+    """A population of one collects, keeps episode statistics and samples exactly as SAC does."""
+    cfg = SACConfig(buffer_size=3 * 4, learning_starts=1000, seed=1)
+    sac, pop = SAC(_TaggedEnv(n=3, obs_dim=6), cfg), SACPopulation(_TaggedEnv(n=3, obs_dim=6), [cfg])
+    for _ in range(11):                          # wraps the 4-slot ring
+        sac._vec_step()
+        pop._vec_step()
+    for key in sac.rb:
+        assert torch.equal(sac.rb[key], pop.rb[key]), key
+    assert (sac.pos, sac.full, sac.num_timesteps) == (pop.pos, pop.full, pop.num_timesteps) == (3, True, 33)
+    assert torch.equal(sac._ep, pop._ep) and pop._ep[0, 3].item() == 3
+    mine, theirs = pop.sample(500), sac.sample(500)
+    for key in theirs:
+        assert torch.equal(mine[key][0], theirs[key]), key
+
+
+def test_evaluate_matches_sb3_quota_restatement_per_agent():
+    pop = SACPopulation(_host_env(2 * 2), [SACConfig(seed=3), SACConfig(seed=4)])
+    refs = _sb3_evaluate(pop.predict, _host_env(2 * 3, seed=9), 5, agents=2)    # quotas 1, 2, 2 per agent
+    ev = pop.evaluate(_host_env(2 * 3, seed=9), 5)
+    assert ev["episodes"] == [5, 5] and refs[0] != refs[1]
+    for k, ref in enumerate(refs):
+        _assert_eval_matches({key: v[k] for key, v in ev.items()}, ref)
 
 
 def test_short_learn_on_the_kernel_body():
