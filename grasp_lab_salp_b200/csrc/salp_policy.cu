@@ -10,6 +10,11 @@
 // value = critic(obs).  The standard-normal `noise` is an input (the caller's torch generator keeps
 // the stream reproducible and CUDA-graph capturable).
 //
+// Deterministic mode (SB3 predict(deterministic=True)): noise == NULL gives action = mean exactly and
+// clipped = the Box clip of the mean; logp may then be NULL (not written).  value == NULL skips the
+// critic (its weights are not even staged), so an evaluation pass does half the work.  With noise
+// given, logp and value are mandatory and the stochastic path is the one above, unchanged.
+//
 // Weights arrive as ONE packed float array (ppo.MlpPolicy.packed()):
 //   actor : W1 [H, D] b1 [H]  W2 [H, H] b2 [H]  W3 [A, H] b3 [A]
 //   critic: W1 [H, D] b1 [H]  W2 [H, H] b2 [H]  W3 [1, H] b3 [1]
@@ -80,9 +85,11 @@ salp_mlp_act_kernel(const float* __restrict__ weights, const float* __restrict__
   stage_segment(sw, weights, o.aW1, g.aW1, MLP_H * D); stage_segment(sw, weights, o.ab1, g.ab1, MLP_H);
   stage_segment(sw, weights, o.aW2, g.aW2, MLP_H * MLP_H); stage_segment(sw, weights, o.ab2, g.ab2, MLP_H);
   stage_segment(sw, weights, o.aW3, g.aW3, MLP_A * MLP_H); stage_segment(sw, weights, o.ab3, g.ab3, MLP_A);
-  stage_segment(sw, weights, o.cW1, g.cW1, MLP_H * D); stage_segment(sw, weights, o.cb1, g.cb1, MLP_H);
-  stage_segment(sw, weights, o.cW2, g.cW2, MLP_H * MLP_H); stage_segment(sw, weights, o.cb2, g.cb2, MLP_H);
-  stage_segment(sw, weights, o.cW3, g.cW3, MLP_H); stage_segment(sw, weights, o.cb3, g.cb3, 1);
+  if (value) {
+    stage_segment(sw, weights, o.cW1, g.cW1, MLP_H * D); stage_segment(sw, weights, o.cb1, g.cb1, MLP_H);
+    stage_segment(sw, weights, o.cW2, g.cW2, MLP_H * MLP_H); stage_segment(sw, weights, o.cb2, g.cb2, MLP_H);
+    stage_segment(sw, weights, o.cW3, g.cW3, MLP_H); stage_segment(sw, weights, o.cb3, g.cb3, 1);
+  }
   stage_segment(sw, weights, o.log_std, g.log_std, MLP_A);
   __syncthreads();
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -100,14 +107,18 @@ salp_mlp_act_kernel(const float* __restrict__ weights, const float* __restrict__
     float m = sw[o.ab3 + a];
 #pragma unroll
     for (int k = 0; k < MLP_H; k++) m = fmaf(sw[o.aW3 + a * MLP_H + k], h[k], m);
-    const float ls = sw[o.log_std + a];
-    const float z = noise[i * MLP_A + a];
-    const float act = fmaf(z, expf(ls), m);
+    float act = m;                                         // deterministic: the mean itself
+    if (noise) {
+      const float ls = sw[o.log_std + a];
+      const float z = noise[i * MLP_A + a];
+      act = fmaf(z, expf(ls), m);
+      lp += -0.5f * z * z - ls - 0.918938533204672742f;    // log(2 pi) / 2
+    }
     action[i * MLP_A + a] = act;
     clipped[i * MLP_A + a] = fminf(fmaxf(act, lo[a]), hi[a]);
-    lp += -0.5f * z * z - ls - 0.918938533204672742f;      // log(2 pi) / 2
   }
-  logp[i] = lp;
+  if (logp) logp[i] = lp;
+  if (!value) return;
   // critic
   mlp_trunk<MAXD>(sw, o.cW1, o.cb1, o.cW2, o.cb2, D, x, h);
   float v = sw[o.cb3];
@@ -123,9 +134,9 @@ int64_t salp_mlp_packed_size(int32_t obs_dim) { return mlp_offsets(obs_dim).tota
 int salp_mlp_act(const float* weights_dev, int32_t obs_dim, const float* obs_dev, const float* noise_dev, int64_t n,
                  const float* action_low, const float* action_high, float* action_dev, float* clipped_dev,
                  float* logp_dev, float* value_dev, void* stream) {
-  if (!weights_dev || !obs_dev || !noise_dev || !action_dev || !clipped_dev || !logp_dev || !value_dev || n <= 0 ||
-      !action_low || !action_high)
+  if (!weights_dev || !obs_dev || !action_dev || !clipped_dev || n <= 0 || !action_low || !action_high)
     return SALP_ERR_INVALID;
+  if (noise_dev && (!logp_dev || !value_dev)) return SALP_ERR_INVALID;    // the rollout needs both
   if (obs_dim < 1 || obs_dim > SALP_OBS_BASE + 2 * SALP_MAX_OBSTACLES) return SALP_ERR_INVALID;
   const MlpOffsets o = mlp_offsets(obs_dim, 4);
   const size_t smem = sizeof(float) * (size_t)o.total;

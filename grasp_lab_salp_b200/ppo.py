@@ -18,6 +18,11 @@ algebra here) and ``SalpBatch.step_device`` all work on device tensors; per-iter
 are reduced on device and read back once.  Multi-GPU: one process per GPU, envs sharded
 (``distributed.make_shard``), gradients and rollout statistics all-reduced over NCCL.
 
+Both algorithms have SB3's ``predict``, ``evaluate`` (evaluate_policy(deterministic=True), also run by
+``learn`` every ``eval_every`` env-steps on an ``eval_env``), ``save`` and ``load`` (torch.save, not SB3's
+zip format).  Inference and evaluation use buffers of their own, so they can run between the captured
+CUDA graphs of a training run without changing it.
+
 The env is anything with ``num_envs``, ``obs_dim``, ``reset_t() -> obs`` and
 ``step_t(actions) -> (obs, reward, terminated, truncated, terminal_obs)`` on torch tensors;
 ``DeviceEnv`` adapts a SalpBatch (CUDA), ``HostEnv`` adapts any numpy backend with the SalpBatch
@@ -33,6 +38,7 @@ import numpy as np
 import torch
 import torch.nn as nn
 
+from .evaluation import run_episodes
 from .params import sort_by_k_auto
 
 
@@ -220,6 +226,7 @@ class PPO:
         self.gen.manual_seed(self._gen_seed)
         self.low = torch.tensor(self.cfg.action_low, device=self.device)
         self.high = torch.tensor(self.cfg.action_high, device=self.device)
+        self._predict_gen = None                    # stochastic predict(): its own stream, never self.gen
         self._fused = None
         if (self.cfg.fused_policy and self.device.type == "cuda" and isinstance(self.policy, MlpPolicy)
                 and tuple(self.cfg.hidden) == (64, 64)):
@@ -479,8 +486,13 @@ class PPO:
         is the same number everywhere even when the shards differ in size."""
         return self.env_steps // self.env.num_envs * self.global_envs
 
-    def learn(self, total_env_steps: int, log=None) -> PPOStats:
+    def learn(self, total_env_steps: int, log=None, eval_env=None, eval_every=0, n_eval_episodes=10) -> PPOStats:
+        """Collect and update until env_steps_global >= total_env_steps, one row of statistics per iteration to
+        `log`.  With an `eval_env` and `eval_every` > 0, the iteration that reaches the next multiple of
+        `eval_every` env-steps runs `evaluate` after its update and its row gains eval_return, eval_success,
+        eval_length and eval_seconds (SB3 EvalCallback).  Evaluation leaves the training state untouched."""
         stats = PPOStats()
+        next_eval = self.env_steps_global + eval_every if eval_env is not None and eval_every > 0 else None
         while self.env_steps_global < total_env_steps:
             t0 = time.perf_counter()
             roll = self.collect()
@@ -501,12 +513,160 @@ class PPO:
             row = dict(iteration=self.iteration, env_steps=self.env_steps_global, mean_step_reward=mean_rew,
                        episodes=n_ep, mean_episode_return=mean_ret, mean_episode_length=mean_len, success_rate=succ,
                        rollout_seconds=t1 - t0, update_seconds=t2 - t1, **upd)
+            if next_eval is not None and self.env_steps_global >= next_eval:
+                t3 = time.perf_counter()
+                ev = self.evaluate(eval_env, n_eval_episodes)
+                row.update(eval_return=ev["mean_return"], eval_success=ev["success_rate"],
+                           eval_length=ev["mean_length"], eval_seconds=time.perf_counter() - t3)
+                while next_eval <= self.env_steps_global:
+                    next_eval += eval_every
             stats.history.append(row)
             for k, v in row.items():
                 setattr(stats, k, v)
             if log:
                 log(row)
         return stats
+
+    # ---- inference ----
+    def _clip(self, a):
+        return torch.minimum(torch.maximum(a, self.low), self.high)
+
+    def _predict_state(self, n, state):
+        """The policy state predict() starts from: none for the MLP policy."""
+        return None
+
+    def _actor_fn(self, n):
+        """The deterministic actor for batches of up to n envs with the weights as they are now (packed once,
+        here): f(obs [k, D] contiguous fp32, episode_start [k] bool or None, state) -> (mean, mean clipped to
+        the Box).  Buffers are its own, so nothing the rollout or its CUDA graphs read is written.  On CUDA the
+        MLP runs as salp_mlp_act in its deterministic mode (no noise, no critic)."""
+        fz = self._fused
+        if fz is None:
+            def f(obs, starts, state):
+                mean = self.policy.actor(obs)
+                return mean, self._clip(mean)
+            return f
+        C, lib, D = fz["C"], fz["lib"], self.env.obs_dim
+        packed = self.policy.packed()
+        mean, clipped = torch.empty((n, 3), device=self.device), torch.empty((n, 3), device=self.device)
+
+        def f(obs, starts, state):
+            k = obs.shape[0]
+            rc = lib.salp_mlp_act(C.c_void_p(packed.data_ptr()), D, C.c_void_p(obs.data_ptr()), None, k, fz["lo"],
+                                  fz["hi"], C.c_void_p(mean.data_ptr()), C.c_void_p(clipped.data_ptr()), None, None,
+                                  C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream))
+            if rc != 0:
+                raise RuntimeError(f"salp_mlp_act failed ({rc})")
+            return mean[:k], clipped[:k]
+        return f
+
+    @torch.no_grad()
+    def predict(self, obs, state=None, episode_start=None, deterministic=False):
+        """stable-baselines3 predict: (actions [N, 3] clipped to the Box, state) for obs [N, obs_dim].  The action
+        is the Gaussian mean (deterministic) or a sample drawn from predict's own generator.  `state` and
+        `episode_start` matter for RecurrentPPO only (the MLP policy returns state None)."""
+        obs = torch.as_tensor(obs, dtype=torch.float32, device=self.device).contiguous()
+        if obs.dim() != 2 or obs.shape[1] != self.env.obs_dim:
+            raise ValueError(f"obs must be [N, {self.env.obs_dim}]")
+        n = obs.shape[0]
+        starts = None if episode_start is None else torch.as_tensor(episode_start, dtype=torch.bool,
+                                                                     device=self.device).reshape(n).contiguous()
+        state = self._predict_state(n, state)
+        mean, clipped = self._actor_fn(n)(obs, starts, state)
+        if not deterministic:
+            if self._predict_gen is None:
+                self._predict_gen = torch.Generator(device=self.device)
+                self._predict_gen.manual_seed(self.cfg.seed + 2)
+            noise = torch.randn(mean.shape, device=self.device, generator=self._predict_gen)
+            clipped = self._clip(mean + noise * self.policy.log_std.exp())
+        return clipped.clone(), state
+
+    def _shard_span(self, n):
+        """(offset of this rank's first env, envs over all ranks) of an eval env sharded over the ranks."""
+        if self.dist_world == 1:
+            return 0, n
+        import torch.distributed as dist
+        sizes = [torch.zeros(1, dtype=torch.int64, device=self.device) for _ in range(self.dist_world)]
+        dist.all_gather(sizes, torch.tensor([n], dtype=torch.int64, device=self.device))
+        sizes = [int(x) for x in sizes]
+        return sum(sizes[:dist.get_rank()]), sum(sizes)
+
+    @torch.no_grad()
+    def evaluate(self, env, n_episodes=10):
+        """Deterministic episodes on `env` (SB3 evaluate_policy(deterministic=True)): env i contributes
+        (n_episodes + i) // N episodes; success is `terminated`.  RecurrentPPO starts every env from a zero
+        actor state and resets it where an episode ended.  Under torch.distributed each rank steps its shard
+        (distributed.make_shard), i counts globally, and every rank returns the same mean_return, mean_length,
+        success_rate and episodes.  The env may step up to 15 times past the last recorded episode."""
+        n = env.num_envs
+        offset, total = self._shard_span(n)
+        quotas = (n_episodes + offset + torch.arange(n, device=env.device)) // total
+        f, state = self._actor_fn(n), self._predict_state(n, None)
+        sums = run_episodes(lambda obs, starts: f(obs.to(self.device).contiguous(), starts, state)[1], env, quotas)
+        if self.dist_world > 1:
+            import torch.distributed as dist
+            dist.all_reduce(sums)
+        r, ln, s, e = sums[0].tolist()
+        return dict(mean_return=r / e, mean_length=ln / e, success_rate=s / e, episodes=int(e))
+
+    # ---- persistence ----
+    def _policy_spec(self):
+        p = self.policy
+        lstm = getattr(p, "lstm_hidden", None)
+        return dict(kind="RecurrentPPO" if lstm else "PPO", obs_dim=self.env.obs_dim, lstm_hidden=lstm,
+                    hidden=tuple(m.out_features for m in p.actor if isinstance(m, nn.Linear))[:-1])
+
+    def save(self, path):
+        """torch.save (not SB3's zip format) of the policy's state_dict, the Adam state, env_steps (over all
+        ranks), iteration, the policy kind and sizes, and per rank the exploration generator state and the
+        reward-normalisation statistics.  Under torch.distributed every rank calls it; rank 0 writes."""
+        mine = dict(gen=self.gen.get_state(), ret_stats=self._ret_stats.cpu())
+        ranks, rank = [mine], 0
+        if self.dist_world > 1:
+            import torch.distributed as dist
+            ranks, rank = [None] * self.dist_world, dist.get_rank()
+            dist.all_gather_object(ranks, mine)
+        if rank == 0:
+            torch.save(dict(spec=self._policy_spec(), policy=self.policy.state_dict(), opt=self.opt.state_dict(),
+                            env_steps=self.env_steps_global, iteration=self.iteration, ranks=ranks), path)
+        if self.dist_world > 1:
+            dist.barrier()
+
+    def load(self, path):
+        """Restore what `save` wrote; training then goes on from a reset env, as SB3's learn does after load.
+        Parameters are copied in place.  Each rank gets back its own generator state and reward-normalisation
+        statistics when the checkpoint was written by as many ranks as there are now; otherwise those keep
+        what the constructor set.  Captured CUDA graphs are dropped (the optimiser state they read is
+        replaced) and captured again by the next rollout and update.  A checkpoint of another policy kind,
+        obs_dim or size raises ValueError."""
+        ck = torch.load(path, map_location="cpu", weights_only=False)
+        if ck["spec"] != self._policy_spec():
+            raise ValueError(f"checkpoint policy {ck['spec']} does not match this one {self._policy_spec()}")
+        self.policy.load_state_dict(ck["policy"])
+        self.opt.load_state_dict(ck["opt"])
+        for g in self.opt.param_groups:           # keep this object's mode, whichever mode wrote the file
+            g["capturable"] = self.use_graphs
+        for st in self.opt.state.values():
+            st["step"] = st["step"].to(self.device) if self.use_graphs else st["step"].cpu()
+        ranks = ck["ranks"]
+        if len(ranks) == self.dist_world:
+            import torch.distributed as dist
+            mine = ranks[dist.get_rank() if self.dist_world > 1 else 0]
+            self.gen.set_state(mine["gen"])
+            self._ret_stats.copy_(mine["ret_stats"])
+        self.env_steps = ck["env_steps"] * self.env.num_envs // self.global_envs
+        self.iteration = ck["iteration"]
+        self._roll_graph = self._upd_graph = None
+        self._roll_calls = self._upd_calls = 0
+        self.opt.zero_grad(set_to_none=True)
+        self._reset_rollout_state()
+
+    def _reset_rollout_state(self):
+        """A reset env and zeroed per-env episode state (what SB3's learn starts from after load)."""
+        self.obs.copy_(self.env.reset_t())
+        self._ep_ret.zero_()
+        self._ep_len.zero_()
+        self._disc_ret.zero_()
 
 
 # ------------------------------------------------------------------------------------------------
@@ -580,6 +740,58 @@ class RecurrentPPO(PPO):
             n = env.num_envs
             self._lstm_fused = dict(actor=LstmCellB200(self.policy.lstm_actor, n), critic=LstmCellB200(self.policy.lstm_critic, n),
                                     h=torch.empty((n, 256), device=self.device), c=torch.empty((n, 256), device=self.device))
+        self._eval_cell = None      # predict / evaluate's own actor cell: the rollout graph reads the rollout cells
+
+    def _predict_state(self, n, state):
+        """The actor LSTM's (h, c) predict() starts from: zeros, or a contiguous copy of the caller's."""
+        if state is None:
+            return tuple(torch.zeros(n, self.policy.lstm_hidden, device=self.device) for _ in range(2))
+        return tuple(torch.as_tensor(x, dtype=torch.float32, device=self.device).reshape(n, -1).clone(
+            memory_format=torch.contiguous_format) for x in state)
+
+    def _actor_fn(self, n):
+        """As PPO._actor_fn for the actor LSTM and its head (sb3_contrib predict: the critic LSTM is not run);
+        `state` = (h, c) is advanced in place, rows with episode_start reset first.  On CUDA the cell is an
+        LstmCellB200 of this function's own, built for up to n envs and packed here."""
+        actor = self.policy.actor
+        if self._lstm_fused is None:
+            cell = self.policy.lstm_actor
+
+            def f(obs, starts, state):
+                h, c = state
+                if starts is not None:
+                    keep = (1.0 - starts.float()).unsqueeze(-1)
+                    h2, c2 = cell(obs, (h * keep, c * keep))
+                else:
+                    h2, c2 = cell(obs, (h, c))
+                h.copy_(h2)
+                c.copy_(c2)
+                mean = actor(h)
+                return mean, self._clip(mean)
+            return f
+        from .lstm import LstmCellB200
+        if self._eval_cell is None or self._eval_cell.n < n:
+            self._eval_cell = LstmCellB200(self.policy.lstm_actor, n)
+        cell = self._eval_cell
+        cell.pack()
+
+        def f(obs, starts, state):
+            cell.step(obs, starts, *state)
+            mean = actor(state[0])
+            return mean, self._clip(mean)
+        return f
+
+    def _reset_rollout_state(self):
+        super()._reset_rollout_state()
+        for x in self.state:
+            x.zero_()
+        self.starts.fill_(True)
+
+    def load(self, path):
+        super().load(path)
+        if self._lstm_fused is not None:
+            self._lstm_fused["actor"].pack()
+            self._lstm_fused["critic"].pack()
 
     def _policy_step(self, obs, starts):
         """One rollout step of the policy on self.state (updated in place): (action mean, value)."""

@@ -58,6 +58,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from . import _lib
+from .evaluation import run_episodes
 
 HIDDEN = 256
 ACT_DIM = 3
@@ -510,29 +511,9 @@ class _SACDriver:
         K, N = self.num_agents, env.num_envs
         if N % K:
             raise ValueError(f"the eval env's num_envs ({N}) must be a multiple of the population size ({K})")
-        m, dev = N // K, env.device
-        targets = ((n_episodes + torch.arange(m, device=dev)) // m).repeat(K)
-        counts = torch.zeros(N, dtype=torch.long, device=dev)
-        sums = torch.zeros((K, 4), dtype=torch.float64, device=dev)        # return, length, successes, episodes
-        cur_r = torch.zeros(N, dtype=torch.float64, device=dev)
-        cur_l = torch.zeros(N, dtype=torch.float64, device=dev)
-        obs = env.reset_t()
-        step = 0
-        while step % 16 or bool((counts < targets).any()):                # (a finished env records nothing more)
-            a = self.predict(obs.float(), deterministic=True)
-            obs, rew, term, trunc, _ = env.step_t(a)
-            t = term.bool()
-            d = t | trunc.bool()
-            cur_r += torch.nan_to_num(rew, nan=0.0, posinf=0.0, neginf=0.0).double()
-            cur_l += 1
-            rec = d & (counts < targets)
-            w = rec.double()
-            sums += torch.stack([cur_r * w, cur_l * w, t.double() * w, w], dim=1).view(K, m, 4).sum(1)
-            counts += rec.long()
-            cur_r.masked_fill_(d, 0.0)
-            cur_l.masked_fill_(d, 0.0)
-            step += 1
-        s = sums.tolist()
+        m = N // K
+        quotas = ((n_episodes + torch.arange(m, device=env.device)) // m).repeat(K)
+        s = run_episodes(lambda obs, starts: self.predict(obs, deterministic=True), env, quotas, K).tolist()
         return dict(mean_return=[x[0] / x[3] for x in s], mean_length=[x[1] / x[3] for x in s],
                     success_rate=[x[2] / x[3] for x in s], episodes=[int(x[3]) for x in s])
 

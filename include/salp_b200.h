@@ -308,7 +308,10 @@ int salp_debug_p4_stamps(long long* out16);
  * W1[64,D] b1[64] W2[64,64] b2[64] W3[1,64] b3[1], log_std[3] (row-major like torch's nn.Linear.weight);
  * salp_mlp_packed_size(D) floats.  noise_dev: standard-normal [N,3].  Outputs: action [N,3] = mean +
  * noise * exp(log_std), clipped [N,3] = action clipped to [low, high] (what the env gets), logp [N], value [N].
- * action_low / action_high: host float[3]. */
+ * action_low / action_high: host float[3].
+ * Deterministic mode (SB3 predict(deterministic=True)): noise_dev NULL gives action = mean exactly, clipped =
+ * the mean clipped to [low, high]; logp_dev may then be NULL (not written).  value_dev NULL skips the critic.
+ * With noise_dev given, logp_dev and value_dev are mandatory. */
 int64_t salp_mlp_packed_size(int32_t obs_dim);
 int salp_mlp_act(const float* weights_dev, int32_t obs_dim, const float* obs_dev, const float* noise_dev, int64_t n,
                  const float* action_low, const float* action_high, float* action_dev, float* clipped_dev,

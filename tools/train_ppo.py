@@ -6,7 +6,10 @@ batched GPU simulator -- BASELINE configs 3 and 4.
     torchrun --nproc-per-node 8 tools/train_ppo.py --envs 65536 ...      (envs = whole job, sharded)
 
 Writes one JSON line per PPO iteration (env_steps, mean step reward, mean episode return /
-length, success rate, approx KL, wall seconds for rollout and update).
+length, success rate, approx KL, wall seconds for rollout and update).  With --eval-every, the iteration
+that reaches each multiple of it also runs a deterministic evaluation on a separate env (eval_return,
+eval_success, eval_length, eval_seconds); --save-best keeps the model with the best eval_return so far
+(SB3 EvalCallback's best_model_save_path), --save writes the final model, --load resumes from a file.
 """
 import argparse
 import json
@@ -22,6 +25,23 @@ from grasp_lab_salp_b200.distributed import make_shard, world_info  # noqa: E402
 from grasp_lab_salp_b200.ppo import PPO, DeviceEnv, PPOConfig, RecurrentPPO  # noqa: E402
 
 
+class FreshEnv:
+    """An eval env rebuilt from its seed at every reset: every evaluation meets the same scenes, so that
+    evaluations during training compare like with like and a saved model's evaluation can be repeated in
+    another process (--evaluate-only)."""
+
+    def __init__(self, make):
+        self.make, self.env = make, make()
+        self.num_envs, self.obs_dim, self.device = self.env.num_envs, self.env.obs_dim, self.env.device
+
+    def reset_t(self):
+        self.env = self.make()
+        return self.env.reset_t()
+
+    def step_t(self, actions):
+        return self.env.step_t(actions)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--envs", type=int, default=16384)
@@ -33,6 +53,14 @@ def main():
     ap.add_argument("--precision", choices=["mixed", "f64"], default="mixed")
     ap.add_argument("--recurrent", action="store_true", help="RecurrentPPO, LSTM(256) actor and critic (config 4)")
     ap.add_argument("--cuda-graphs", action="store_true", help="replay rollout and minibatch steps as CUDA graphs")
+    ap.add_argument("--eval-every", type=int, default=0, help="env-steps between deterministic evaluations")
+    ap.add_argument("--eval-envs", type=int, default=64)
+    ap.add_argument("--eval-episodes", type=int, default=64)
+    ap.add_argument("--save", default=None, help="write the final model here (torch.save)")
+    ap.add_argument("--save-best", default=None, help="write the model with the best eval_return so far here")
+    ap.add_argument("--load", default=None, help="resume from a file written by --save / --save-best")
+    ap.add_argument("--evaluate-only", action="store_true",
+                    help="with --load: evaluate the loaded model once on the eval env, print the result and exit")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     rank, local, world = world_info()
@@ -46,10 +74,22 @@ def main():
     algo = RecurrentPPO if args.recurrent else PPO
     ppo = algo(DeviceEnv(batch), PPOConfig(n_steps=args.n_steps, n_epochs=args.n_epochs, batch_size=args.batch_size,
                                            seed=args.seed, cuda_graphs=args.cuda_graphs))
+    if args.load:
+        ppo.load(args.load)
+    eval_env = FreshEnv(lambda: DeviceEnv(make_shard(args.eval_envs, params, seed=10_000 + args.seed)))
+    if args.evaluate_only:
+        ev = ppo.evaluate(eval_env, args.eval_episodes)
+        if rank == 0:
+            print(json.dumps(dict(ev, evaluate_only=True, load=args.load)), flush=True)
+        return
     out = open(args.out, "w") if (args.out and rank == 0) else None
     t0 = time.perf_counter()
+    best = [float("-inf")]
 
     def log(row):
+        if args.save_best and "eval_return" in row and row["eval_return"] > best[0]:
+            best[0] = row["eval_return"]
+            ppo.save(args.save_best)               # (every rank: save gathers the per-rank state)
         if rank == 0:
             row = dict(row, wall_seconds=time.perf_counter() - t0)
             line = json.dumps(row)
@@ -58,8 +98,12 @@ def main():
                 out.write(line + "\n")
                 out.flush()
 
-    stats = ppo.learn(args.total_steps, log=log)
+    stats = ppo.learn(args.total_steps, log=log, eval_env=eval_env if args.eval_every else None,
+                      eval_every=args.eval_every, n_eval_episodes=args.eval_episodes)
     batch.check()
+    if args.save:
+        ppo.save(args.save)
+    evals = [h for h in stats.history if "eval_return" in h]
     ar = ppo.allreduce_seconds_per_step()
     if rank == 0:
         wall = time.perf_counter() - t0
@@ -76,7 +120,10 @@ def main():
                           "wall_seconds": wall, "env_steps_per_sec_incl_learner": stats.env_steps / wall,
                           "env_steps_per_sec_rollout_only": stats.env_steps / sim,
                           "final_success_rate": stats.success_rate,
-                          "final_mean_episode_return": stats.mean_episode_return}), flush=True)
+                          "final_mean_episode_return": stats.mean_episode_return,
+                          "final_eval_success": evals[-1]["eval_success"] if evals else None,
+                          "final_eval_return": evals[-1]["eval_return"] if evals else None,
+                          "eval_seconds_total": sum(h["eval_seconds"] for h in evals)}), flush=True)
     if world > 1:
         # (no destroy_process_group(): with NCCL collectives captured in CUDA graphs it blocked at exit on
         #  8 GPUs; leave at once instead)
