@@ -116,6 +116,164 @@ TOL_MIXED = dict(rtol=1e-5, floor=0.1, small_floor=0.1, accel_rtol=1e-4, accel_f
                  obs_floor=0.1, metric_floor=0.1)
 
 
+# ---------------------------------------------------------------------------------------------
+# coefficient sets off make_env()'s configuration
+# ---------------------------------------------------------------------------------------------
+# make_derived (csrc/salp_loop_mixed.cuh) gives the loop its axisymmetric form (SalpDerived.axisym)
+# when these eight conditions hold on the fp32 roundings of the coefficients; make_env()'s defaults
+# satisfy all of them.  AXISYM_CONDITIONS names them, axisym_broken() restates the predicate.
+AXISYM_CONDITIONS = ("Ca", "Cat", "Car01", "Car12", "thi", "tspan", "rhi", "rspan")
+
+
+def axisym_broken(p):
+    """The conditions of the axisymmetric-form predicate that `p` breaks (empty: the AXI form),
+    compared on fp32 roundings exactly as make_derived does."""
+    f = np.float32
+    ca = [f(x) for x in p.added_mass_force]
+    cat = [f(x) for x in p.added_mass_torque]
+    car = [f(x) for x in p.added_mass_rate_force]
+    t, r = list(p.trans_drag_range), list(p.rot_drag_range)
+    thi = [f(t[2 * i + 1]) for i in range(3)]
+    tspan = [f(t[2 * i + 1] - t[2 * i]) for i in range(3)]
+    rhi = [f(r[2 * i + 1]) for i in range(3)]
+    rspan = [f(r[2 * i + 1] - r[2 * i]) for i in range(3)]
+    holds = {"Ca": ca[1] == ca[2], "Cat": cat[1] == cat[2], "Car01": car[0] == car[1], "Car12": car[1] == car[2],
+             "thi": thi[1] == thi[2], "tspan": tspan[1] == tspan[2], "rhi": rhi[1] == rhi[2], "rspan": rspan[1] == rspan[2]}
+    return {k for k in AXISYM_CONDITIONS if not holds[k]}
+
+
+def asymmetric_params(precision, num_obstacles=2):
+    """Every coefficient family behind the axisymmetric-form predicate distinct per axis (so the
+    roll and pitch rates are driven at real amplitude, 1e-3 rad/s, not by rounding noise), on a
+    body that is not make_env()'s either: sea-water density, a heavier and longer body, another
+    nozzle, other penalties."""
+    p = golden_params(load_golden("ref_random.npz"), precision=precision, num_obstacles=num_obstacles)
+    p.density = 1025.0
+    p.dry_mass = 1.3
+    p.init_length = 0.34
+    p.init_width = 0.16
+    p.nozzle_length1 = 0.04
+    p.nozzle_length2 = 0.06
+    p.nozzle_area = 0.0002
+    p.nozzle_mass = 0.8
+    p.discharge_coefficient = 0.35
+    p.drag_force_ratio = 0.2
+    p.added_mass_force[:] = [0.45, 0.65, 0.55]
+    p.added_mass_torque[:] = [0.25, 0.5, 0.7]
+    p.added_mass_rate_force[:] = [0.15, 0.2, 0.25]
+    p.trans_drag_range[:] = [1.4, 2.6, 2.4, 1.6, 2.7, 1.3]
+    p.rot_drag_range[:] = [0.12, 0.28, 0.45, 0.25, 0.55, 0.15]
+    p.target_radius = 0.25
+    p.max_cycles = 40
+    assert axisym_broken(p) == set(AXISYM_CONDITIONS)
+    return p
+
+
+def one_break(name, precision=None, num_obstacles=2):
+    """make_env()'s defaults with exactly ONE condition of the axisymmetric-form predicate broken
+    (AXISYM_CONDITIONS): each reaches a different subset of the general form's extra terms."""
+    from grasp_lab_salp_b200 import PRECISION_MIXED
+    p = golden_params(load_golden("ref_random.npz"), precision=PRECISION_MIXED if precision is None else precision,
+                      num_obstacles=num_obstacles)
+    # defaults: Ca (0.5, 0.6, 0.6), Cat (0.3, 0.6, 0.6), Car 0.2, trans (lo, hi) per axis (1.5, 2.5) (2.5, 1.5)
+    # (2.5, 1.5), rot (0.1, 0.3) (0.5, 0.2) (0.5, 0.2)
+    if name == "Ca":
+        p.added_mass_force[2] = 0.7
+    elif name == "Cat":
+        p.added_mass_torque[2] = 0.75
+    elif name == "Car01":
+        p.added_mass_rate_force[0] = 0.15
+    elif name == "Car12":
+        p.added_mass_rate_force[2] = 0.25
+    elif name == "thi":            # same span, another upper end
+        p.trans_drag_range[4:6] = [2.75, 1.75]
+    elif name == "tspan":          # same upper end, another span
+        p.trans_drag_range[4] = 2.75
+    elif name == "rhi":
+        p.rot_drag_range[4:6] = [0.75, 0.45]
+    elif name == "rspan":
+        p.rot_drag_range[4] = 0.625
+    else:
+        raise KeyError(name)
+    assert axisym_broken(p) == {name}, (name, axisym_broken(p))
+    return p
+
+
+# Per-channel floors of the 1e-5 per-step tolerance on asymmetric_params() and the one_break() sets.
+# MIXED_FLOORS was measured where roll and pitch are rounding noise; here they are driven (roll rate
+# ~2e-3 rad/s, pitch rate through zero at real amplitude), so the out-of-plane channels need other
+# floors.  "needed" = the smallest floor with which every sample holds 1e-5 (largest |a - b| / 1e-5
+# over the samples that fail the pure relative test), measured on the host build of the fused body
+# (256 envs x 8 steps) and on a B200 (pipeline kernel at 1000 and 6001 envs, fused and fused
+# K-sorted kernels; 1000 envs x 8 steps), with the action mix of test_gpu_configurations.edge_actions
+# (uniform and clipped-Gaussian, K = 0 rows, short cycles, auto-reset), obstacle counts 0, 1, 8 and
+# the eight one_break sets.  Floors are 2-3x the worse of the two:
+#                      needed: host    B200
+ASYM_FLOORS = {
+    "posw_x": 0.2,     # 7.4e-2  9.4e-2
+    "posw_y": 0.2,     # 6.4e-2  7.2e-2
+    "pos_x": 0.15,     # 5.9e-2  4.8e-2
+    "pos_y": 0.03,     # 6.3e-3  1.1e-2
+    "vel_x": 0.04,     # 7.9e-3  1.7e-2
+    "vel_y": 0.02,     # 4.2e-3  7.6e-3
+    "euler_z": 0.2,    # 7.6e-2  8.1e-2
+    "angle_z": 0.2,    # 5.2e-2  7.5e-2
+    "angvel_z": 6e-3,  # 2.4e-3  2.7e-3
+    "posw_z": 2e-4,    # 6.5e-5  7.7e-5
+    "vel_z": 1e-5,     # 3.1e-6  3.8e-6
+    "euler_x": 4.5e-4,     # 1.5e-4  1.8e-4
+    "euler_y": 4e-4,   # 1.1e-4  1.6e-4
+    "angvel_x": 1e-6,  # 2.6e-7  4.5e-7
+    "angvel_y": 2.5e-5,    # 9.3e-6  8.6e-6
+    "length": 1e-9, "width": 1e-9, "prev_volume": 1e-9, "com_x": 1e-9,     # 0 (identical bits: fp64 in both)
+    "prev_dist": 1e-3,     # 0  0
+}
+
+
+def tumbling(n, seed=100):
+    """inject= of lockstep_compare: a tumbling body before every step -- roll and pitch rates up to
+    0.3 rad/s, vertical velocity up to 0.1 m/s.  Left to themselves roll and pitch stay near 1e-3
+    rad/s, where the general form's terms in w0 w1, w1 w2 and v1 v2 move the state by less than fp32
+    noise: a swapped axis index there (CatF[2] for CatF[1] in JdI[2]) passes a per-step tolerance.
+    Tumbling, they act at real amplitude: the same fault then moves the position by 1e-3 m in one
+    step, 100x the per-step tolerance."""
+    def inject(t):
+        rng = np.random.default_rng(seed + t)
+        # (roll and pitch restart within 0.3 rad: a cycle then stays clear of the pitch = +-pi/2
+        #  singularity of the Euler rates, where fp32 and fp64 trajectories part for good reason)
+        return {"angvel_x": rng.uniform(-0.3, 0.3, n), "angvel_y": rng.uniform(-0.3, 0.3, n),
+                "vel_z": rng.uniform(-0.1, 0.1, n), "euler_x": rng.uniform(-0.3, 0.3, n),
+                "euler_y": rng.uniform(-0.3, 0.3, n)}
+    return inject
+
+
+# Floors for tumbling() steps: roll, pitch and z now move at in-plane amplitudes, and so do their
+# errors.  Measured like ASYM_FLOORS, on asymmetric_params() and the one_break() sets:
+#                      needed: host    B200
+TUMBLING_FLOORS = {
+    "posw_x": 0.25,    # 1.1e-1  5.1e-2
+    "posw_y": 0.2,     # 5.8e-2  8.8e-2
+    "pos_x": 0.12,     # 3.6e-2  4.6e-2
+    "pos_y": 0.02,     # 8.0e-3  8.3e-3
+    "vel_x": 0.04,     # 6.5e-3  1.6e-2
+    "vel_y": 0.02,     # 7.0e-3  5.3e-3
+    "euler_z": 0.25,   # 4.8e-2  1.1e-1
+    "angle_z": 0.15,   # 5.4e-2  6.9e-2
+    "angvel_z": 3e-3,  # 1.3e-3  1.0e-3
+    "posw_z": 0.04,    # 1.8e-2  1.7e-2
+    "vel_z": 1e-3,     # 3.7e-4  2.6e-4
+    "euler_x": 0.1,    # 4.2e-2  4.4e-2
+    "euler_y": 0.08,   # 3.5e-2  2.9e-2
+    "angvel_x": 0.012,     # 2.4e-3  5.6e-3
+    "angvel_y": 4e-3,  # 6.8e-4  1.7e-3
+    "length": 1e-9, "width": 1e-9, "prev_volume": 1e-9, "com_x": 1e-9,     # 0 (identical bits: fp64 in both)
+    "prev_dist": 1e-3,     # 0  0
+}
+# The reward (float64 total, relative to max(|r|, floor)) off the defaults, free and tumbling: needed
+# 10.6 and 11.5 on the B200, below MIXED's 10 on the host build.
+ASYM_REWARD_FLOOR = 30.0
+
+
 def replay_golden(backend, g, rtol, *, small_rtol=None, small_floor=1e-7, floor=1e-9, accel_rtol=None,
                   accel_floor=1e-6, reward_floor=1e-3, obs_floor=1e-4, metric_floor=1e-6,
                   check_metrics=True, report=None, regular_tilt=None):
@@ -272,7 +430,7 @@ def obs_errors(got, ref, floor, tag):
 
 
 def lockstep_compare(product, oracle, actions, *, resync, rtol, floor, reward_floor=10.0, obs_floor=0.1,
-                     small_floor=None, num_obstacles=2, report=None, floors=None):
+                     small_floor=None, num_obstacles=2, report=None, floors=None, inject=None):
     """Step `product` and `oracle` with the same actions [T,N,3] (auto-reset on, same scenes).
 
     Bit-exact: K, cycle, phase, terminated, truncated (hence the reset indices), episode index.
@@ -281,6 +439,8 @@ def lockstep_compare(product, oracle, actions, *, resync, rtol, floor, reward_fl
     comparison is a single env-step from identical state (the per-step tolerance);
     resync=False lets both run free (long-horizon drift; returns the error history instead of
     asserting on floats).
+    inject: optional callable(t) -> {column: values}, written into both backends before step t
+    (after the resync), e.g. tumbling().
     """
     T = actions.shape[0]
     obs_p = product.reset().copy()
@@ -296,6 +456,9 @@ def lockstep_compare(product, oracle, actions, *, resync, rtol, floor, reward_fl
                 if col in skip:
                     continue
                 product.set_state(col, oracle.get_state(col))
+        for col, v in (inject(t) if inject is not None else {}).items():
+            product.set_state(col, v)
+            oracle.set_state(col, v)
         a = actions[t]
         obs_p, rew_p, term_p, trunc_p = product.step(a, auto_reset=True)
         obs_o, rew_o, term_o, trunc_o = oracle.step(a, auto_reset=True)

@@ -6,7 +6,9 @@ import pytest
 from emu_backend import EmuBatch, emu_cdll, emu_lane_cdll
 from grasp_lab_salp_b200 import PRECISION_F64, PRECISION_MIXED
 from oracle.salp_oracle import OracleVecEnv
-from parity import check_blowup_golden, TOL_F64, MIXED_FLOORS, TOL_MIXED, TOL_MIXED_FREE_RUN, golden_params, lockstep_compare, sample_scene_pool, load_golden, replay_golden
+from parity import (check_blowup_golden, ASYM_FLOORS, AXISYM_CONDITIONS, TOL_F64, MIXED_FLOORS, TOL_MIXED, TOL_MIXED_FREE_RUN,
+                    asymmetric_params, axisym_broken, golden_params, lockstep_compare, one_break, sample_scene_pool, load_golden,
+                    replay_golden, tumbling, TUMBLING_FLOORS)
 
 GOLDENS = ["ref_fixed10.npz", "ref_edge.npz", "ref_random.npz", "ref_clipped.npz"]
 
@@ -139,32 +141,53 @@ def test_other_obstacle_counts(num_obstacles):
 
 def test_non_default_robot_parameters():
     """Nothing is hard-wired to make_env()'s literals: sea-water density, a heavier and longer body,
-    another nozzle, other penalties -- fp32 kernel body vs oracle, per-step tolerance."""
-    g = load_golden("ref_random.npz")
+    another nozzle, other penalties, and every added-mass and drag family distinct per axis (the
+    general form of the loop, roll and pitch driven at real amplitude) -- kernel body vs oracle,
+    per-step tolerance with the floors measured for this set (ASYM_FLOORS)."""
     n, T = 48, 8
-    for prec, tol in ((PRECISION_F64, dict(rtol=1e-9, floor=1e-3)), (PRECISION_MIXED, dict(rtol=1e-5, floor=0.1))):
-        p = golden_params(g, precision=prec)
-        p.density = 1025.0
-        p.dry_mass = 1.3
-        p.init_length = 0.34
-        p.init_width = 0.16
-        p.nozzle_length1 = 0.04
-        p.nozzle_length2 = 0.06
-        p.nozzle_area = 0.0002
-        p.nozzle_mass = 0.8
-        p.discharge_coefficient = 0.35
-        p.drag_force_ratio = 0.2
-        p.added_mass_force[:] = [0.45, 0.65, 0.55]
-        p.added_mass_torque[:] = [0.25, 0.5, 0.7]
-        p.trans_drag_range[:] = [1.4, 2.6, 2.4, 1.6, 2.7, 1.3]
-        p.rot_drag_range[:] = [0.12, 0.28, 0.45, 0.25, 0.55, 0.15]
-        p.target_radius = 0.25
-        p.max_cycles = 40
-        prod, orc = EmuBatch(n, p, seed=11), OracleVecEnv(n, p, seed=11)
-        acts = np.random.default_rng(5).uniform([0.1, 0, -1], [1, 1, 1], size=(T, n, 3)).astype(np.float32)
-        report = {}
-        lockstep_compare(prod, orc, acts, resync=True, report=report, **tol)
-        print(prec, max(report.values()))
+    for tumble in (False, True):
+        for prec, tol in ((PRECISION_F64, dict(rtol=1e-9, floor=1e-3)),
+                          (PRECISION_MIXED, dict(rtol=TOL_MIXED["rtol"], floor=TOL_MIXED["floor"],
+                                                 floors=TUMBLING_FLOORS if tumble else ASYM_FLOORS))):
+            p = asymmetric_params(prec)
+            prod, orc = EmuBatch(n, p, seed=11), OracleVecEnv(n, p, seed=11)
+            acts = np.random.default_rng(5).uniform([0.1, 0, -1], [1, 1, 1], size=(T, n, 3)).astype(np.float32)
+            report = {}
+            lockstep_compare(prod, orc, acts, resync=True, report=report, inject=tumbling(n) if tumble else None, **tol)
+            print(prec, "tumbling" if tumble else "free", report)
+            assert np.abs(orc.get_state("angvel_x")).max() > 1e-4     # roll is driven, not rounding noise
+
+
+def test_axisymmetric_form_predicate():
+    """parity.axisym_broken restates make_derived's predicate: the defaults take the AXI form,
+    asymmetric_params() breaks all eight conditions, each one_break() set exactly its own."""
+    assert axisym_broken(golden_params(load_golden("ref_random.npz"))) == set()
+    assert axisym_broken(asymmetric_params(PRECISION_MIXED)) == set(AXISYM_CONDITIONS)
+    for name in AXISYM_CONDITIONS:
+        assert axisym_broken(one_break(name)) == {name}
+    # fp32 roundings, not the doubles: an axis-2 value one fp64 ulp off is still the AXI form
+    p = golden_params(load_golden("ref_random.npz"))
+    p.added_mass_force[2] = np.nextafter(p.added_mass_force[1], 1.0)
+    assert axisym_broken(p) == set()
+
+
+@pytest.mark.parametrize("tumble", [False, True], ids=["free", "tumbling"])
+@pytest.mark.parametrize("name", AXISYM_CONDITIONS)
+@pytest.mark.parametrize("precision", [PRECISION_F64, PRECISION_MIXED])
+def test_one_broken_axisymmetry_condition(precision, name, tumble):
+    """The defaults with one condition of the axisymmetric-form predicate broken: the general form
+    of the loop against the oracle, per step, free and from a tumbling state (parity.tumbling)."""
+    n, T = 48, 4
+    p = one_break(name, precision)
+    prod, orc = EmuBatch(n, p, seed=12), OracleVecEnv(n, p, seed=12)
+    acts = np.random.default_rng(6).uniform([0, 0, -1], [1, 1, 1], size=(T, n, 3)).astype(np.float32)
+    if precision == PRECISION_F64:
+        tol = dict(rtol=1e-9, floor=1e-3)
+    else:
+        tol = dict(rtol=TOL_MIXED["rtol"], floor=TOL_MIXED["floor"], floors=TUMBLING_FLOORS if tumble else ASYM_FLOORS)
+    report = {}
+    lockstep_compare(prod, orc, acts, resync=True, report=report, inject=tumbling(n) if tumble else None, **tol)
+    print(name, precision, report)
 
 
 def test_masked_reset_and_zero_substep_cycles():
