@@ -147,19 +147,33 @@ int salp_launch_step(const SalpParams& p, const SalpView& v, const SalpStepIO& i
     if (dev < 0 || dev >= 64 || !configured4[dev]) {
       SalpParams widest = p;
       widest.num_obstacles = SALP_MAX_OBSTACLES;
-      const int bytes = (int)pipe4_smem_bytes(widest, false);
-      if (cudaFuncSetAttribute(salp_step_kernel_pipe4<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes) != cudaSuccess ||
-          cudaFuncSetAttribute(salp_step_kernel_pipe4<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes) != cudaSuccess)
+      const int bytes = (int)pipe4_smem_bytes(widest, false, false);
+      const int bytes_wide = (int)pipe4_smem_bytes(widest, false, true);
+      if (cudaFuncSetAttribute(salp_step_kernel_pipe4<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes) != cudaSuccess ||
+          cudaFuncSetAttribute(salp_step_kernel_pipe4<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes) != cudaSuccess ||
+          cudaFuncSetAttribute(salp_step_kernel_pipe4<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes_wide) != cudaSuccess ||
+          cudaFuncSetAttribute(salp_step_kernel_pipe4<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes_wide) != cudaSuccess)
         return SALP_ERR_CUDA;
       if (dev >= 0 && dev < 64) configured4[dev] = true;
     }
-    const uint32_t pflags = (flags & 0x3fffffffu) | (grid_for(v.n, 32) > sms ? SALP_P4_FLAG_SHARED_SM : 0u);
-    if (flags & SALP_STEP_CHECK_HANDOFF)      // (a separate kernel: the production one keeps its register allocation)
-      salp_step_kernel_pipe4<true><<<grid_for(v.n, 32), SALP_P4_THREADS, pipe4_smem_bytes(p, dv.axisym != 0), stream>>>(
-          p, dv, v, io, pflags, order);
+    // One block per SM (<= #SMs blocks): the 8-warp form, whose four producer warps hand the dyn warp
+    // whole coefficient sets (salp_pipe4_kernel.cuh).  SALP_PIPE_WIDE=0 forces the 4-warp form there
+    // (experiment switch; read at every launch so that one process can compare the two).
+    const bool shared_sm = grid_for(v.n, 32) > sms;
+    const char* wide_env = getenv("SALP_PIPE_WIDE");
+    const bool wide = !shared_sm && !(wide_env && atoi(wide_env) == 0);
+    const uint32_t pflags = (flags & 0x3fffffffu) | (shared_sm ? SALP_P4_FLAG_SHARED_SM : 0u);
+    const dim3 grid((unsigned)grid_for(v.n, 32));
+    const size_t smem = pipe4_smem_bytes(p, dv.axisym != 0, wide);
+    const bool check = (flags & SALP_STEP_CHECK_HANDOFF) != 0;   // (a separate kernel: the production one keeps its register allocation)
+    if (wide && check)
+      salp_step_kernel_pipe4<true, true><<<grid, SALP_P4W_THREADS, smem, stream>>>(p, dv, v, io, pflags, order);
+    else if (wide)
+      salp_step_kernel_pipe4<false, true><<<grid, SALP_P4W_THREADS, smem, stream>>>(p, dv, v, io, pflags, order);
+    else if (check)
+      salp_step_kernel_pipe4<true, false><<<grid, SALP_P4_THREADS, smem, stream>>>(p, dv, v, io, pflags, order);
     else
-      salp_step_kernel_pipe4<false><<<grid_for(v.n, 32), SALP_P4_THREADS, pipe4_smem_bytes(p, dv.axisym != 0), stream>>>(
-          p, dv, v, io, pflags, order);
+      salp_step_kernel_pipe4<false, false><<<grid, SALP_P4_THREADS, smem, stream>>>(p, dv, v, io, pflags, order);
     name = "salp_step_kernel_pipe4";
     SALP_LAUNCH_CHECK();
     return launches + 1;

@@ -34,7 +34,13 @@
 // co-resident blocks per SM interleave their roles over the sub-partitions).
 //
 // Envs may be visited through a permutation (`order`, the K-sort).
+//
+// With one block per SM (<= #SMs x 32 envs) the launcher runs the 8-warp form (WIDE): four producer warps
+// compute whole coefficient sets for every fourth chunk, side by side in time, and the dyn warp only loads
+// them (see the producer branch below; DESIGN.md 3.2).
 #pragma once
+#include <type_traits>
+
 #include "salp_pipe_kernel.cuh"
 
 #define SALP_P4_CHUNK 8
@@ -68,9 +74,65 @@ struct P4Layout {
   static constexpr size_t tags = snap + 2 * (sizeof(float4) * 5 * 32 + sizeof(double2) * 3 * 32);   // [SLOTS1 + SLOTS2 + SLOTS3][32] int (checked mode)
   static constexpr size_t tile = tags + sizeof(int) * (SALP_P4_SLOTS1 + SALP_P4_SLOTS2 + SALP_P4_SLOTS3) * 32;   // [2][32][D] float
 };
-static inline size_t pipe4_smem_bytes(const SalpParams& p, bool axi) {
+
+// The wide form (one block per SM, 8 warps): the four producer warps each compute WHOLE coefficient
+// sets (shape_front + make_coefs) for every fourth chunk, into ring C: one slot of 8 rows per
+// producer, rows of five quads (axisymmetric form) or seven, stored as planes of quads.  Rings 1 and
+// 2 do not exist in this form, so ring C's full / empty barriers take their ids (1..8); ring 3 keeps
+// its own (11..14).
+#define SALP_P4W_THREADS 256
+#define SALP_P4W_PRODUCERS 4
+#define SALP_P4W_SLOTSC (SALP_P4_CHUNK * SALP_P4W_PRODUCERS)
+#define P4W_FULLC(b) (1 + (b))
+#define P4W_EMPTYC(b) (1 + SALP_P4W_PRODUCERS + (b))
+static_assert(P4W_EMPTYC(SALP_P4W_PRODUCERS - 1) < P4_FULL3(0), "ring C's barriers must not reach ring 3's");
+template <bool AXI>
+struct P4WLayout {
+  static constexpr int QC = AXI ? 5 : 7;                                                       // quads per ring-C row (whole Coef32)
+  static constexpr size_t ringC = 0;                                                           // [SLOTSC][QC][32] float4
+  static constexpr size_t ring3a = ringC + sizeof(float4) * SALP_P4W_SLOTSC * QC * 32;
+  static constexpr size_t ring3b = ring3a + sizeof(float4) * SALP_P4_SLOTS3 * 32;
+  static constexpr size_t merge = ring3b + sizeof(float2) * SALP_P4_SLOTS3 * 32;
+  static constexpr size_t snap = merge + sizeof(double) * SALP_P4_MERGE * 32;
+  static constexpr size_t tags = snap + 2 * (sizeof(float4) * 5 * 32 + sizeof(double2) * 3 * 32);   // [SLOTSC + SLOTS3][32] int (checked mode)
+  static constexpr size_t tile = tags + sizeof(int) * (SALP_P4W_SLOTSC + SALP_P4_SLOTS3) * 32;
+};
+static inline size_t pipe4_smem_bytes(const SalpParams& p, bool axi, bool wide) {
   const size_t tile = sizeof(float) * 2 * 32 * (SALP_OBS_BASE + 2 * p.num_obstacles);
+  if (wide) return (axi ? P4WLayout<true>::tile : P4WLayout<false>::tile) + tile;
   return (axi ? P4Layout<true>::tile : P4Layout<false>::tile) + tile;
+}
+// whole coefficient set of one substep, as read by dyn_step<false, false, AXI> (inv_m / inv_Iz are
+// only read by the disturbance variant, which never runs in this kernel)
+template <bool AXI>
+__device__ __forceinline__ void coef_store_full(const Coef32& g, float4* row) {
+  row[0] = make_float4(g.aj[0], g.aj[1], g.aj[2], g.com);
+  row[32] = make_float4(g.kdm[0], g.kdm[1], g.xc[0], g.xc[1]);
+  row[64] = make_float4(g.com_rate2, g.com_acc, g.tj1, g.tj2);
+  row[96] = make_float4(g.kqI[0], g.kqI[1], g.klI[0], g.klI[1]);
+  if (AXI) {
+    row[128] = make_float4(g.JdI[1], g.AdI[1], 0.f, 0.f);
+  } else {
+    row[128] = make_float4(g.JdI[0], g.JdI[1], g.JdI[2], g.AdI[0]);
+    row[160] = make_float4(g.AdI[1], g.AdI[2], g.kdm[2], g.xc[2]);
+    row[192] = make_float4(g.kqI[2], g.klI[2], 0.f, 0.f);
+  }
+}
+template <bool AXI>
+__device__ __forceinline__ void coef_load_full(Coef32& g, const float4* row) {
+  const float4 a = row[0], b = row[32], c = row[64], d = row[96], e = row[128];
+  g.aj[0] = a.x; g.aj[1] = a.y; g.aj[2] = a.z; g.com = a.w;
+  g.kdm[0] = b.x; g.kdm[1] = b.y; g.xc[0] = b.z; g.xc[1] = b.w;
+  g.com_rate2 = c.x; g.com_acc = c.y; g.tj1 = c.z; g.tj2 = c.w;
+  g.kqI[0] = d.x; g.kqI[1] = d.y; g.klI[0] = d.z; g.klI[1] = d.w;
+  if (AXI) {
+    g.JdI[1] = e.x; g.AdI[1] = e.y;
+  } else {
+    const float4 f = row[160], h = row[192];
+    g.JdI[0] = e.x; g.JdI[1] = e.y; g.JdI[2] = e.z; g.AdI[0] = e.w;
+    g.AdI[1] = f.x; g.AdI[2] = f.y; g.kdm[2] = f.z; g.xc[2] = f.w;
+    g.kqI[2] = h.x; g.klI[2] = h.y;
+  }
 }
 
 // Iterations j = j0..je of one hand-off chunk, for ALL lanes and without any lane test: a full chunk
@@ -131,15 +193,24 @@ __device__ long long salp_p4_stamps[16];
     if ((flags & SALP_P4_FLAG_STAMPS) && blockIdx.x == 0 && warp == 0 && lane == 0) salp_p4_stamps[k] = clock64(); \
   } while (0)
 
-template <bool AXI, bool CHECK>
+template <bool AXI, bool CHECK, bool WIDE>
 __device__ __forceinline__ void salp_pipe4_body(const SalpParams& p, const SalpDerived& dv, const SalpView& v,
                                                 const SalpStepIO& io, uint32_t flags, const int32_t* __restrict__ order,
                                                 unsigned char* smem) {
-  using L = P4Layout<AXI>;
-  constexpr int Q2 = L::Q2;
+  using L = std::conditional_t<WIDE, P4WLayout<AXI>, P4Layout<AXI>>;
+  constexpr int Q2 = P4Layout<AXI>::Q2;
+  constexpr int QC = P4WLayout<AXI>::QC;
   constexpr int C = SALP_P4_CHUNK;
-  float4* ring2 = reinterpret_cast<float4*>(smem + L::ring2);
-  float4* ring1 = reinterpret_cast<float4*>(smem + L::ring1);
+  constexpr int NP = SALP_P4W_PRODUCERS;
+  float4* ring1 = nullptr;
+  float4* ring2 = nullptr;
+  float4* ringC = nullptr;
+  if constexpr (WIDE) {
+    ringC = reinterpret_cast<float4*>(smem + L::ringC);
+  } else {
+    ring2 = reinterpret_cast<float4*>(smem + L::ring2);
+    ring1 = reinterpret_cast<float4*>(smem + L::ring1);
+  }
   float4* ring3a = reinterpret_cast<float4*>(smem + L::ring3a);
   float2* ring3b = reinterpret_cast<float2*>(smem + L::ring3b);
   double* merge = reinterpret_cast<double*>(smem + L::merge);
@@ -147,9 +218,9 @@ __device__ __forceinline__ void salp_pipe4_body(const SalpParams& p, const SalpD
   float4* snap_kin = snap_dyn + 5 * 32;                                          // [5][32]
   double2* tot_dyn = reinterpret_cast<double2*>(snap_kin + 5 * 32);             // [3][32]
   double2* tot_kin = tot_dyn + 3 * 32;                                           // [3][32]
-  int* tags1 = reinterpret_cast<int*>(smem + L::tags);
+  int* tags1 = reinterpret_cast<int*>(smem + L::tags);          // (wide form: ring C's tags)
   int* tags2 = tags1 + SALP_P4_SLOTS1 * 32;
-  int* tags3 = tags2 + SALP_P4_SLOTS2 * 32;
+  int* tags3 = WIDE ? tags1 + SALP_P4W_SLOTSC * 32 : tags2 + SALP_P4_SLOTS2 * 32;
   float* tile = reinterpret_cast<float*>(smem + L::tile);
   const int lane = threadIdx.x & 31;
   // Role of this warp: 0 dyn, 1 kin, 2 coefs R, 3 front, one per SM sub-partition.  With two blocks
@@ -175,6 +246,29 @@ __device__ __forceinline__ void salp_pipe4_body(const SalpParams& p, const SalpD
     const int base = seen == 15 ? slot_of_warp[widx] : widx;
     warp = (base + 2 * (int)(ticket & 1u)) & 3;
   }
+  if constexpr (WIDE) {
+    // Eight warps, two per sub-partition.  Roles by sub-partition (hardware slot %warpid & 3, as above):
+    // the dyn warp shares its sub-partition with the idle warp only, so it issues alone; kin shares
+    // with the other idle warp (it trails dyn at ~82 cycles per substep and must keep pace); the four
+    // producers fill the other two sub-partitions.  Roles: 0 dyn, 1 kin, 2..5 producers, 6 / 7 idle.
+    // If the slots do not come out two per sub-partition, the roles follow threadIdx.x instead.
+    __shared__ int hw_slot[8];
+    unsigned hw;
+    asm volatile("mov.u32 %0, %%warpid;" : "=r"(hw));
+    if (lane == 0) hw_slot[widx] = (int)(hw & 3u);
+    __syncthreads();
+    unsigned counts = 0;                           // four 4-bit counters, one per sub-partition
+    int rank = 0;
+#pragma unroll
+    for (int w = 0; w < 8; w++) {
+      counts += 1u << (4 * hw_slot[w]);
+      if (w < widx && hw_slot[w] == hw_slot[widx]) rank++;
+    }
+    const bool paired = counts == 0x2222u;
+    const int sub = paired ? hw_slot[widx] : (widx & 3), r = paired ? rank : (widx >> 2);
+    warp = sub >= 2 ? 2 + 2 * (sub - 2) + r : (r ? 6 + sub : sub);   // {0 dyn, 6} {1 kin, 7} {2, 3} {4, 5}
+  }
+  const bool idle = WIDE && warp >= 2 + NP;
   const int64_t tid = (int64_t)blockIdx.x * 32 + lane;
   const bool live = tid < v.n;
   const int64_t i = live ? (order ? (int64_t)order[tid] : tid) : 0;
@@ -187,7 +281,7 @@ __device__ __forceinline__ void salp_pipe4_body(const SalpParams& p, const SalpD
   int Kraw = 0;
   PhasePlan pp;
   pp.k_ref = pp.k_T0 = pp.k_jet = pp.upd_a_end = pp.upd_b_begin = pp.upd_b_end = 0;
-  if (live) {
+  if (live && !idle) {
     env_step_begin(p, v, io, i, cx, b);
     P4_STAMP(1);
     Kraw = plan_substeps(cx.plan, v.time_table);
@@ -207,16 +301,79 @@ __device__ __forceinline__ void salp_pipe4_body(const SalpParams& p, const SalpD
   const int nch3 = Kw > 1 ? (Kw - 1 + C - 1) / C : 0;
   const float dir[3] = {(float)cx.plan.dir[0], (float)cx.plan.dir[1], (float)cx.plan.dir[2]};
   P4_STAMP(2);
-  if ((flags & SALP_P4_FLAG_STAMPS) && blockIdx.x == 0 && warp == 0 && lane == 0) { salp_p4_stamps[8] = Kw; salp_p4_stamps[9] = Wmax; }
+  if ((flags & SALP_P4_FLAG_STAMPS) && blockIdx.x == 0 && warp == 0 && lane == 0) {
+    salp_p4_stamps[8] = Kw; salp_p4_stamps[9] = Wmax; salp_p4_stamps[10] = blockDim.x;   // (blockDim: which form ran)
+  }
   // ring rows of substep j (planes of quads)
   auto row1 = [&](int j) { return ring1 + (j % SALP_P4_SLOTS1) * 2 * 32 + lane; };
   auto row2 = [&](int j) { return ring2 + (j % SALP_P4_SLOTS2) * Q2 * 32 + lane; };
+  auto rowC = [&](int j) { return ringC + (j % SALP_P4W_SLOTSC) * QC * 32 + lane; };
   auto put_tag = [&](int* plane, int slots, int j) { if (CHECK) plane[(j % slots) * 32 + lane] = j; };
   auto check_tag = [&](const int* plane, int slots, int j, bool mine = true) {     // mine: a row was produced for this lane
     if (CHECK && mine && plane[(j % slots) * 32 + lane] != j) raise_status(v, SALP_ERR_HANDOFF);
   };
 
-  if (warp == 3) {
+  if (WIDE && warp >= 2) {
+    // ---------------- wide form: producer f computes whole coefficient sets for chunks c = f mod NP ----------------
+    // Every coefficient set depends on the action and the substep index only, so the producers work
+    // side by side in time.  Each one seeds its fp64 shape track at the first substep j0 of a chunk by
+    // running the two updates before it (j0 - 2 sets the centre of mass, j0 - 1 the carried rate; every
+    // other field the later updates read is a pure function of t_j), with t_j from the table, which
+    // holds the same chain of additions as the carried sum.  tests/test_emu_shape_seed.py checks that
+    // the seeded track gives the bits of the carried one.  The seeding updates go through the same two
+    // inlined shape_front calls as the others, with all their outputs live: a copy whose ShapeFront is
+    // discarded was measured to contract its fp64 arithmetic differently (one ulp of the centre of
+    // mass).  make_coefs is the fused kernel's arithmetic.
+    if (!idle) {
+      const int f = warp - 2;
+      ShapeTrack st;
+      if (K > 0) {
+        Coef32 g0;
+        mixed_init_shape<AXI>(p, dv, b, dir, st, g0);
+      }
+      for (int c = f; c < nch2; c += NP) {
+        const int j0 = c * C + 1;
+        const int je = (c + 1) * C < Wmax ? (c + 1) * C : Wmax;
+        auto one = [&](double tj, int j) {
+          ShapeFront fr;
+          shape_front(p, dv, cx.plan, tj, j, pp.k_T0, pp.k_jet, st, fr);
+          if (j >= j0) {
+            Coef32 g;
+            make_coefs<AXI>(dv, dir, fr, g);
+            coef_store_full<AXI>(g, rowC(j));
+            put_tag(tags1, SALP_P4W_SLOTSC, j);
+          }
+        };
+        if (c >= NP) pipe_bar_sync(P4W_EMPTYC(f));
+        // (a lane whose updates end at j0 - 2 or j0 - 1 seeds part-way: its last update belongs to the
+        //  previous chunk, hence to another producer, whose track stays untouched)
+        const int js = c > 0 ? j0 - 2 : j0;
+        double tj = v.time_table[js];
+        for (int j = js; j <= je; j += 2) {      // two updates per trip (independent chains, as in the front warp)
+          const double tj1 = rn::dadd(tj, p.dt);
+          if (j + 1 <= je && j + 1 <= kA) {
+            one(tj, j);
+            one(tj1, j + 1);
+          } else if (j <= kA) {
+            one(tj, j);
+          }
+          tj = rn::dadd(tj1, p.dt);
+        }
+        __syncwarp();
+        pipe_bar_arrive(P4W_FULLC(f));
+      }
+      // the fp64 shape columns of a lane come from the producer that ran its last update (chunk 0's
+      // producer for a lane without one)
+      const int last_chunk = kA > 0 ? (kA - 1) / C : 0;
+      if (K > 0 && last_chunk % NP == f) {
+        mixed_finish_shape(p, st, K, b);
+        merge[0 * 32 + lane] = b.length; merge[1 * 32 + lane] = b.width; merge[2 * 32 + lane] = b.prev_volume;
+        merge[3 * 32 + lane] = b.prevI[0]; merge[4 * 32 + lane] = b.prevI[1];
+        merge[5 * 32 + lane] = b.com; merge[6 * 32 + lane] = b.com_rate; merge[7 * 32 + lane] = b.prev_com_rate;
+        merge[8 * 32 + lane] = b.com_acc;
+      }
+    }
+  } else if (!WIDE && warp == 3) {
     // ---------------- front: fp64 shape chain + backward differences, j = 1..kA ----------------
     // ring 1 has TWO readers (coefs R and dyn): a buffer is free when both have arrived (96 threads);
     // "full" is signalled to coefs R only -- the dyn warp reads chunk c after ring 2's chunk c is full
@@ -272,7 +429,7 @@ __device__ __forceinline__ void salp_pipe4_body(const SalpParams& p, const SalpD
       merge[5 * 32 + lane] = b.com; merge[6 * 32 + lane] = b.com_rate; merge[7 * 32 + lane] = b.prev_com_rate;
       merge[8 * 32 + lane] = b.com_acc;
     }
-  } else if (warp == 2) {
+  } else if (!WIDE && warp == 2) {
     // ---------------- coefs R: the rotational half of the coefficient set of each ShapeFront ----------------
     auto one = [&](int j) {
       ShapeFront f;
@@ -379,14 +536,32 @@ __device__ __forceinline__ void salp_pipe4_body(const SalpParams& p, const SalpD
     }
     P4_STAMP(3);
     // g_j: translational half computed here from the ShapeFront (independent of the motion state: it
-    // fills the latency shadows of the recurrence), rotational half from ring 2
+    // fills the latency shadows of the recurrence), rotational half from ring 2.  Wide form: the whole
+    // set from ring C.
     auto coefs_of = [&](int j) {
-      ShapeFront f;
-      front_load(f, row1(j));
-      coef_load_R<AXI>(g, row2(j));
-      check_tag(tags1, SALP_P4_SLOTS1, j, j < K);             // (the producers stop at each lane's own K)
-      check_tag(tags2, SALP_P4_SLOTS2, j, j < K);
-      make_coefs_T<AXI>(dv, dir, f, g);
+      if constexpr (WIDE) {
+        coef_load_full<AXI>(g, rowC(j));
+        check_tag(tags1, SALP_P4W_SLOTSC, j, j < K);          // (the producers stop at each lane's own K)
+      } else {
+        ShapeFront f;
+        front_load(f, row1(j));
+        coef_load_R<AXI>(g, row2(j));
+        check_tag(tags1, SALP_P4_SLOTS1, j, j < K);
+        check_tag(tags2, SALP_P4_SLOTS2, j, j < K);
+        make_coefs_T<AXI>(dv, dir, f, g);
+      }
+    };
+    auto wait_coefs = [&](int c) {      // (ring 1 chunk c was full before ring 2 chunk c)
+      if (WIDE) pipe_bar_sync(P4W_FULLC(c % NP));
+      else pipe_bar_sync(P4_FULL2(c % SALP_P4_NBUF2));
+    };
+    auto release_coefs = [&](int c) {
+      if (WIDE) {
+        pipe_bar_arrive(P4W_EMPTYC(c % NP));
+      } else {
+        pipe_bar_arrive(P4_EMPTY1(c % SALP_P4_NBUF1), 96);
+        pipe_bar_arrive(P4_EMPTY2(c % SALP_P4_NBUF2));
+      }
     };
     // snapshot of this warp's per-lane state (18 floats) / fp64 totals, see p4_run_chunk
     auto put_state = [&](bool pr) {
@@ -449,21 +624,19 @@ __device__ __forceinline__ void salp_pipe4_body(const SalpParams& p, const SalpD
     auto chunk_end = [&](int cc) { return (cc + 1) * C < Kw - 1 ? (cc + 1) * C : Kw - 1; };
     const int nA = WA / C < nch3 ? WA / C : nch3;              // chunks with je <= WA (and ring-3 traffic)
     for (; c < nA; c++) {
-      pipe_bar_sync(P4_FULL2(c % SALP_P4_NBUF2));              // (ring 1 chunk c was full before ring 2 chunk c)
+      wait_coefs(c);
       if (c >= SALP_P4_NBUF3) pipe_bar_sync(P4_EMPTY3(c % SALP_P4_NBUF3));
       p4_run_chunk(c * C + 1, (c + 1) * C, dyn_iter_load);
       __syncwarp();
-      pipe_bar_arrive(P4_EMPTY1(c % SALP_P4_NBUF1), 96);
-      pipe_bar_arrive(P4_EMPTY2(c % SALP_P4_NBUF2));
+      release_coefs(c);
       pipe_bar_arrive(P4_FULL3(c % SALP_P4_NBUF3));
     }
     for (; c < nch2; c++) {
-      pipe_bar_sync(P4_FULL2(c % SALP_P4_NBUF2));
+      wait_coefs(c);
       if (c < nch3 && c >= SALP_P4_NBUF3) pipe_bar_sync(P4_EMPTY3(c % SALP_P4_NBUF3));
       p4_run_chunk(c * C + 1, chunk_end(c), dyn_iter_moving);
       __syncwarp();
-      pipe_bar_arrive(P4_EMPTY1(c % SALP_P4_NBUF1), 96);
-      pipe_bar_arrive(P4_EMPTY2(c % SALP_P4_NBUF2));
+      release_coefs(c);
       if (c < nch3) pipe_bar_arrive(P4_FULL3(c % SALP_P4_NBUF3));
     }
     for (; c < nch3 && c < SALP_P4_NBUF3; c++) {               // (only when the shape motion ends within the first chunks)
@@ -530,13 +703,15 @@ __device__ __forceinline__ void salp_pipe4_body(const SalpParams& p, const SalpD
   P4_STAMP(7);
 }
 
-template <bool CHECK>
-__global__ void __launch_bounds__(SALP_P4_THREADS, 2)
+// WIDE: the 8-warp form for one block per SM (launcher: no SALP_P4_FLAG_SHARED_SM); otherwise two
+// 4-warp blocks fit an SM
+template <bool CHECK, bool WIDE>
+__global__ void __launch_bounds__(WIDE ? SALP_P4W_THREADS : SALP_P4_THREADS, WIDE ? 1 : 2)
 salp_step_kernel_pipe4(const __grid_constant__ SalpParams p, const __grid_constant__ SalpDerived dv,
                        const __grid_constant__ SalpView v, const __grid_constant__ SalpStepIO io, uint32_t flags,
                        const int32_t* __restrict__ order) {
   extern __shared__ __align__(16) unsigned char pipe4_smem[];
   // (block-uniform: dv is a kernel argument; both forms give the same bits for axisymmetric parameters)
-  if (dv.axisym) salp_pipe4_body<true, CHECK>(p, dv, v, io, flags, order, pipe4_smem);
-  else salp_pipe4_body<false, CHECK>(p, dv, v, io, flags, order, pipe4_smem);
+  if (dv.axisym) salp_pipe4_body<true, CHECK, WIDE>(p, dv, v, io, flags, order, pipe4_smem);
+  else salp_pipe4_body<false, CHECK, WIDE>(p, dv, v, io, flags, order, pipe4_smem);
 }
